@@ -1,6 +1,7 @@
 """bench.py -- DGG forward+backward throughput (nodes/s) at Pubmed shape on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload pubmed]
+                    [--dump-outputs DIR]
 
 One "step" = one ``DGG.forward`` + backward (gradients for every DGG parameter) over one Pubmed-shape
 graph batch (N=19 717 nodes, F=500, h=64, E~108 k incl. self loops; BASELINE.json configs[2],
@@ -295,14 +296,12 @@ def run_ours(args, rank, local_rank, world):
         dsets.append(dict(adj=adj, x=s["x"].to(dev), g_vals=s["g_vals"].to(dev), g_xenc=s["g_xenc"].to(dev)))
     flat_grads = None
 
-    def eager_step(s, static_grads=False):
+    def eager_step(s):
         for p in params:            # zero_grad(set_to_none=True): the backward's own buffers become the .grad tensors
             p.grad = None           # (no fill, no accumulation kernels); a captured graph returns them as outputs
         out, x_enc = m(s["x"], s["adj"])
         torch.autograd.backward([out._dgg_vals, x_enc], [s["g_vals"], s["g_xenc"]])
-        if static_grads:
-            return out._dgg_vals, [p.grad for p in params]
-        return out._dgg_vals
+        return out._dgg_vals, x_enc, [p.grad for p in params]
 
     # one captured CUDA graph per resident input set (a training loop that holds its mini-batches on the
     # device replays its step); --no-graph times the eager path instead
@@ -326,31 +325,33 @@ def run_ours(args, rank, local_rank, world):
                 grad_sync = "NCCL all_reduce captured in the step graph"
 
         def graph_body(s, j):
-            out, grads = eager_step(s, True)
+            out, x_enc, grads = eager_step(s)
             if world > 1:       # one batched copy instead of a fill + one accumulation kernel per parameter
                 flat = peer_ar[j % 2].buffer if peer_ar is not None else flat_grads
                 torch.cat([g.reshape(-1) for g in grads], out=flat)
                 if peer_ar is not None:
-                    return out, peer_ar[j % 2]()
+                    return out, x_enc, peer_ar[j % 2]()
                 dist.all_reduce(flat)
-                return out, flat
-            return out, grads
+                return out, x_enc, flat
+            return out, x_enc, grads
 
         graphed = []
         for j, s in enumerate(dsets):       # N_SETS is even: consecutive replays alternate between the two buffers
             graphed.append(dgg_b200.GraphedStep(lambda s=s, j=j: graph_body(s, j)))
 
     replay_no = [0]     # a running index (not the caller's): consecutive replays must alternate the gradient buffers
+    last = [None]       # (edge values, x_enc, weight gradients) of the latest step: what --dump-outputs writes
 
     def step_resident(i):
         if graphed is not None:
-            graphed[replay_no[0] % N_SETS]()
+            last[0] = graphed[replay_no[0] % N_SETS]()
             replay_no[0] += 1
         else:
-            eager_step(dsets[i % N_SETS])
+            last[0] = eager_step(dsets[i % N_SETS])
             if world > 1:
                 flat = torch.cat([p.grad.flatten() for p in params])
                 dist.all_reduce(flat)
+                last[0] = last[0][:2] + (flat,)
 
     # ---- host-buffer inputs (the `e2e` arm): what train_small_graphs.py does every call ----
     pinned = [dict(idx=s["idx"].pin_memory(), val=s["val"].pin_memory(), x=s["x"].pin_memory()) for s in host_sets]
@@ -404,6 +405,7 @@ def run_ours(args, rank, local_rank, world):
     l0 = L.dggb_kernel_launches()
     ms = time_region(step_resident, args.steps, world)
     launches = int(L.dggb_kernel_launches() - l0)
+    outputs = step_outputs(last[0], m) if args.dump_outputs and rank == 0 else None
     if graphed is not None:   # replayed graphs launch the kernels recorded at capture time
         launches = sum(graphed[i % N_SETS].dggb_launches_per_replay for i in range(args.steps))
         assert N_SETS % 2 == 0
@@ -471,8 +473,27 @@ def run_ours(args, rank, local_rank, world):
                          h2d_bytes_per_step=int(h2d), d2h_bytes_per_step=int(d2h)),
                 gpu_launches=launches, roofline=roofline, cpu_baseline=cpu, parity=parity, clocks=clocks, epoch=epoch,
                 reddit=reddit)
+    if outputs is not None:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     print(json.dumps(line), flush=True)
     finish(world)
+
+
+def step_outputs(res, m):
+    """What a caller of the timed step receives, copied to the host as float32: the DGG edge values (in the order of
+    the input's coalesced support), x_enc, and every parameter's gradient (summed over the ranks when several GPUs
+    take part).  About 6 MB at Pubmed shape."""
+    vals, x_enc, grads = res
+    named = list(m.named_parameters())
+    if torch.is_tensor(grads):      # one flat all-reduced buffer
+        grads = grads.split([q.numel() for _, q in named])
+    out = dict(out_values=vals, x_enc=x_enc)
+    out.update({f"grad.{k}": g.reshape(q.shape) for (k, q), g in zip(named, grads)})
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
 
 
 def finish(world):
@@ -1214,7 +1235,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="pubmed", choices=["pubmed", "reddit"])
     ap.add_argument("--no-graph", action="store_true", help="time the eager step instead of CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (edge values, x_enc, weight "
+                         "gradients) as DIR/<name>.npy; the inputs depend on the arguments only, so two builds can "
+                         "be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "pubmed"):
+        ap.error("--dump-outputs covers the pubmed workload of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -12,7 +12,7 @@ section 4), so the oracle is pinned against *outputs of the reference modules
 themselves*, run in the build container through ``oracle/ref_loader.py``:
 ``tests/golden/make_golden.py`` stores those outputs as fixtures and
 ``tests/test_oracle_pinned.py`` checks every function here against them (and,
-when ``/root/reference`` is present, against the live reference modules).
+when ``DGG_REFERENCE_ROOT`` names a reference checkout, against the live reference modules).
 The one third-party piece, PyG 2.1.0 ``DenseGraphConv`` (model.py:128-129), has
 no source in the reference tree: ``sage_dense_mean`` restates its published
 semantics -- parity unpinned at that boundary.

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- loader for the *unmodified* reference modules.
 
-Imports ``dgm`` / ``model`` from ``/root/reference`` (read-only, only present in
-the build container, never on the GPU box) through three shims and no source
+Imports ``dgm`` / ``model`` from the reference checkout that ``DGG_REFERENCE_ROOT``
+names (read-only; it is not part of this repository) through three shims and no source
 edits (SURVEY.md section 8c / Appendix C):
 
   1. a stub ``torch_geometric`` registered in ``sys.modules`` (model.py:9-11 and
@@ -24,11 +24,16 @@ import types
 
 import torch
 
-REFERENCE_ROOT = os.environ.get("DGG_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("DGG_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "dgm.py"))
+    """True when ``DGG_REFERENCE_ROOT`` names a reference checkout; a name that points anywhere else is an error."""
+    if not REFERENCE_ROOT:
+        return False
+    if not os.path.isfile(os.path.join(REFERENCE_ROOT, "dgm.py")):
+        raise FileNotFoundError(f"DGG_REFERENCE_ROOT={REFERENCE_ROOT!r} is not a reference checkout (no dgm.py)")
+    return True
 
 
 # --------------------------------------------------------------------------- #
@@ -121,7 +126,7 @@ def load_reference(names=("dgm", "model")):
     """Return the reference modules under private names (``_ref_dgm`` ...) so the
     repo's own drop-in ``dgm`` / ``model`` stay importable next to them."""
     if not reference_available():
-        raise FileNotFoundError(f"reference not found under {REFERENCE_ROOT}")
+        raise FileNotFoundError("no reference checkout: set DGG_REFERENCE_ROOT")
     install_pyg_stub()
     neutralise_cuda()
     out = {}

@@ -1,5 +1,5 @@
 import os, sys, argparse
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch, bench, dgg_b200, model as models
 import torch.nn.functional as F
 from torch.profiler import profile, ProfilerActivity

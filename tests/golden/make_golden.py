@@ -1,9 +1,7 @@
 """Generate the known-answer fixtures under tests/golden/ by running the
-UNMODIFIED reference modules (``/root/reference``) through oracle/ref_loader.py.
+UNMODIFIED reference modules (the checkout ``DGG_REFERENCE_ROOT`` names) through oracle/ref_loader.py:
 
-Run in the build container only (the reference does not exist on the GPU box):
-
-    python tests/golden/make_golden.py
+    DGG_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py
 
 The reference has no tests or golden vectors of its own (SURVEY.md section 4);
 these fixtures are what pins oracle/dgg_oracle.py and, through it, the CUDA path.

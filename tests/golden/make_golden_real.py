@@ -22,6 +22,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 from oracle import ref_loader  # noqa: E402
+from tests.helpers import save_golden_npz  # noqa: E402
 
 warnings.filterwarnings("ignore")
 KEEP_GRADS = 8   # gradients of the first / last few parameters are stored, plus the norm of all of them
@@ -95,8 +96,8 @@ def main():
     fx["citeseer_gcnii_dgg64"] = run(ref, "citeseer_gcnii_dgg64", cs, "GCNII_DGG",
                                      dict(nfeat=cs[1].shape[1], nlayers=64, nhidden=64, nclass=6, dropout=0.6,
                                           lamda=0.5, alpha=0.1, variant=False), a1, seed=42)
-    path = os.path.join(HERE, "real_cora_citeseer.pt")
-    torch.save(fx, path)
+    path = os.path.join(HERE, "real_cora_citeseer.npz")
+    save_golden_npz(path, fx)
     print("wrote", path, os.path.getsize(path) // 1024, "KiB")
 
 

@@ -1,4 +1,46 @@
+import json
+
+import numpy as np
 import torch
+
+
+def save_golden_npz(path, tree):
+    """Nested dicts of tensors (dense or sparse COO), numbers, strings and None -> one compressed .npz that loads
+    without pickle.  Integer tensors are stored in the narrowest dtype that holds their values (the file stays small);
+    ``load_golden_npz`` restores every tensor with its original dtype, bit for bit."""
+    arrays = {}
+
+    def enc(key, v):
+        if isinstance(v, torch.Tensor):
+            if v.is_sparse:
+                v = v.coalesce()
+                return {"sparse": list(v.shape), "indices": enc(key + ".indices", v.indices()),
+                        "values": enc(key + ".values", v.values())}
+            a = v.detach().cpu().numpy()
+            if a.dtype.kind in "iu" and a.size:
+                a = a.astype(np.result_type(np.min_scalar_type(a.min()), np.min_scalar_type(a.max())))
+            arrays[key] = a
+            return {"tensor": key, "dtype": str(v.dtype).split(".")[1]}
+        if isinstance(v, dict):
+            return {"dict": {k: enc(f"{key}/{k}", x) for k, x in v.items()}}
+        return {"value": v}
+
+    meta = enc("", tree)
+    np.savez_compressed(path, __meta__=np.array(json.dumps(meta)), **arrays)
+
+
+def load_golden_npz(path):
+    with np.load(path, allow_pickle=False) as f:
+        def dec(m):
+            if "sparse" in m:
+                return torch.sparse_coo_tensor(dec(m["indices"]), dec(m["values"]), m["sparse"]).coalesce()
+            if "tensor" in m:
+                return torch.from_numpy(f[m["tensor"]]).to(getattr(torch, m["dtype"]))
+            if "dict" in m:
+                return {k: dec(x) for k, x in m["dict"].items()}
+            return m["value"]
+
+        return dec(json.loads(str(f["__meta__"])))
 
 
 def random_graph(n, avg_deg, seed, self_loops=True, hubs=0, hub_deg=0, device="cpu"):

@@ -1,5 +1,6 @@
-"""CPU: checkpoints in the reference's format round-trip through the drop-in modules, and -- where the reference
-checkout exists -- a ``state_dict`` produced by the REFERENCE's own classes loads into them key for key."""
+"""CPU: checkpoints in the reference's format round-trip through the drop-in modules, and a ``state_dict`` produced by
+the REFERENCE's own classes loads into them key for key: live where a reference checkout exists, otherwise from the
+reference state_dicts stored in tests/golden/dgg_golden.pt."""
 import argparse
 import os
 
@@ -42,13 +43,25 @@ def test_checkpoint_round_trip(tmp_path, name):
     assert dgg_b200.checkpoint.load_checkpoint(fn, b) is None
 
 
+# state_dicts of the reference's own classes stored by tests/golden/make_golden.py (tests/golden/dgg_golden.pt)
+GOLDEN_STATE = {"GCN_DGG": "model_gcn_dgg", "GCN_DGG_00": "model_gcn_dgg_00", "GCNII_DGG": "model_gcnii_dgg",
+                "SAGE_DGG": "model_sage_dgg", "SAGE_DGG_00": "model_sage_dgg_00", "GAT_DGG_00": "model_gat_dgg_00"}
+
+
 @pytest.mark.parametrize("name", ["GCN_DGG", "GCN_DGG_00", "GCNII_DGG", "SAGE_DGG", "SAGE_DGG_00", "GAT_DGG_00", "GCN",
                                   "GCNII", "SAGE", "GAT"])
-def test_reference_state_dict_loads(name):
+def test_reference_state_dict_loads(golden, name):
     from oracle import ref_loader
 
     if not ref_loader.reference_available():
-        pytest.skip("reference checkout not present")
+        if name not in GOLDEN_STATE:
+            pytest.skip(f"no stored reference state_dict of {name}: needs a reference checkout (DGG_REFERENCE_ROOT)")
+        g, c = golden["graph"], golden["cases"][GOLDEN_STATE[name]]
+        ours = models.__dict__[name](nfeat=g["f"], nlayers=4, nhidden=g["h"], nclass=g["nclass"], dropout=0.0,
+                                     lamda=0.5, alpha=0.1, variant=False, args=argparse.Namespace(**c["args"]))
+        ours.load_state_dict(c["state"], strict=True)
+        assert {k: v.shape for k, v in ours.state_dict().items()} == {k: v.shape for k, v in c["state"].items()}
+        return
     ref = ref_loader.load_reference(("dgm", "model"))["model"]
     args = _args(extra_edge_dim=2 if name in ("GCN_DGG", "GCNII_DGG", "SAGE_DGG") else 0)
     torch.manual_seed(0)

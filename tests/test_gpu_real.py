@@ -1,5 +1,5 @@
 """GPU parity on the reference's own datasets (BASELINE.json configs[0] and [1]) against outputs of the
-unmodified reference (tests/golden/real_cora_citeseer.pt, made by tests/golden/make_golden_real.py):
+unmodified reference (tests/golden/real_cora_citeseer.npz, made by tests/golden/make_golden_real.py):
 Cora GCN_DGG with injected symmetric Gumbel noise, Citeseer GCNII_DGG with 64 layers.
 
 Weights come from ``torch.manual_seed(seed)`` (the drop-in modules consume the RNG exactly like the reference;
@@ -24,8 +24,10 @@ def _gumbel(shape, seed, scale):
 def real():
     import os
 
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "real_cora_citeseer.pt")
-    return torch.load(path, weights_only=False)
+    from tests.helpers import load_golden_npz
+
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "real_cora_citeseer.npz")
+    return load_golden_npz(path)
 
 
 @pytest.mark.parametrize("tag", ["cora_gcn_dgg", "citeseer_gcnii_dgg64"])

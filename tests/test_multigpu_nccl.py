@@ -1,5 +1,5 @@
 """2-GPU NCCL run of the row-sharded all-pairs DGG path against the unsharded single-GPU result
-(skipped on a 1-GPU box; run with `gpurun --gpus 2 -- python -m pytest tests/test_multigpu_nccl.py`)."""
+(skipped on a machine with fewer than two GPUs)."""
 import os
 
 import pytest

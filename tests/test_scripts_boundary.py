@@ -4,7 +4,7 @@ With ``PYTHONPATH=<repo>:<reference>`` the UNMODIFIED ``train_small_graphs.py``,
 ``train_large_graphs.py`` must import (they do ``from utils import *`` and rely on the reference's whole ``utils``
 namespace, which the repo's ``utils.py`` re-exports), parse their default arguments, and construct every DGG model
 through the string lookup ``models.__dict__[args.model](..., args=args)`` (train_small_graphs.py:387-397) -- against
-THIS repo's ``model.py`` / ``dgm.py``.  Runs only where the reference checkout exists (the build container);
+THIS repo's ``model.py`` / ``dgm.py``.  Runs only where ``DGG_REFERENCE_ROOT`` names a reference checkout;
 ``torch_geometric`` is not installable here, so the test registers the oracle's stub first (test infrastructure)."""
 import os
 import subprocess
@@ -13,10 +13,9 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("DGG_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("DGG_REFERENCE_ROOT", "")
 
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "train_small_graphs.py")),
-                                reason="reference checkout not present")
+pytestmark = pytest.mark.skipif(not REF, reason="no reference checkout (set DGG_REFERENCE_ROOT)")
 
 MODELS = ["GCN_DGG", "GCN_DGG_00", "GCN_DGG_Ablations", "GCN_DGG_00_LargeGraphs", "GCNII_DGG", "SAGE_DGG",
           "SAGE_DGG_00", "GAT_DGG_00", "GAT_DGG_Ablations", "GCN", "GCNII", "SAGE", "GAT"]

@@ -48,7 +48,7 @@ def test_add_noisy_edges_matches_reference_module():
     from oracle import ref_loader
 
     if not ref_loader.reference_available():
-        pytest.skip("reference checkout not present")
+        pytest.skip("no reference checkout (set DGG_REFERENCE_ROOT)")
     ref = ref_loader.load_reference(("utils",))["utils"]
     a = _graph(400, 1500, 3)
     U._NOISY_CACHE.clear()
