@@ -194,7 +194,8 @@ class DGG_LearnableK_SDD(nn.Module):
         return int(self._need_host.item()) > self._kc_last
 
     def _pick_kc(self, k, n):
-        need_dev = torch.ceil(k.detach().max() + self.k_window).clamp(min=1.0)
+        # (never more than the n columns a row has: kc == n already selects every one of them)
+        need_dev = torch.ceil(k.detach().max() + self.k_window).clamp(min=1.0, max=float(n))
         capturing = k.is_cuda and torch.cuda.is_current_stream_capturing()
         if self.exact_kc and not capturing:
             need = int(need_dev.item())

@@ -400,7 +400,7 @@ int dggb_allpairs_topk_fwd(const float* z /* [n,d] */, int32_t n, int32_t d, int
  * dggb_allpairs_topk_fwd, but only entries that sort strictly AFTER (after_val[r], after_idx[r]) -- the last entry
  * the previous pass returned for row r -- in (value descending, column ascending) order are admitted; pass p + 1 of
  * a row therefore returns ranks [64 p, 64 (p + 1)).  after_val / after_idx: [row_count], both or neither NULL.
- * Returns DGGB_ERR_K_OVERFLOW for the d = 128 / 3xTF32 tile shape, which has no continuation kernel. */
+ * A row whose after_idx is -1 (the previous pass ran out of columns) admits nothing: all its slots come back empty. */
 int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d, int32_t row_begin, int32_t row_count,
                                  const float* t, const float* noise, int64_t noise_ld, uint64_t seed,
                                  float noise_scale, int32_t kc, int32_t precision, void* workspace,

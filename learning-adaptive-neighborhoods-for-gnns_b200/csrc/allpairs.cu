@@ -382,8 +382,9 @@ __global__ void __launch_bounds__(kAPThreads, 1)
     const bool wide = kc > 32;
     // continuation pass (rows that need more than 64 entries): only entries that sort strictly AFTER
     // (after_val, after_idx) -- the last entry the previous pass returned for this row -- are admitted
-    const float ubv = (after_val != nullptr && row_ok) ? __ldg(after_val + lrow) : INFINITY;
+    // (an empty last entry, idx -1: the previous pass ran out of columns, so nothing is left to admit)
     const int ubc = (after_idx != nullptr && row_ok) ? __ldg(after_idx + lrow) : -1;
+    const float ubv = (after_val != nullptr && row_ok) ? (ubc < 0 ? -INFINITY : __ldg(after_val + lrow)) : INFINITY;
     auto flush = [&](unsigned need) {
       __syncwarp();   // queue entries were written by their owner lanes; the whole warp reads them below
       while (need) {
@@ -532,7 +533,10 @@ __host__ __device__ inline AP2Smem ap2_smem_layout(int kb, int split, int stages
   return L;
 }
 
-template <int KB, int SPLIT, int NOISE>
+// CONT: the continuation instantiation (d = 65..128 at 3xTF32, where v1 has no tile shape): rows are written with
+// stride out_ld, and when after_val / after_idx are given ([row_count] with stride after_ld) only entries that sort
+// strictly after that entry are admitted -- the predicate of v1's continuation pass.  One column part only.
+template <int KB, int SPLIT, int NOISE, bool CONT = false>
 __global__ void __launch_bounds__(kAP2Threads, 1)
     allpairs_topk2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
                           const float* __restrict__ z_hi, const float* __restrict__ z_lo, int npad, int dpad,
@@ -541,7 +545,8 @@ __global__ void __launch_bounds__(kAP2Threads, 1)
                           unsigned long long seed, float noise_scale, int kc, int stages, int qcap, int qflush,
                           int32_t* __restrict__ out_idx, float* __restrict__ out_val, float inv_temp,
                           float* __restrict__ out_rowsum, int no_prefilter, int tiles_per_part,
-                          int32_t* __restrict__ part_idx, float* __restrict__ part_val) {
+                          int32_t* __restrict__ part_idx, float* __restrict__ part_val, int out_ld,
+                          const float* __restrict__ after_val, const int32_t* __restrict__ after_idx, int after_ld) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
   const AP2Smem L = ap2_smem_layout(KB, SPLIT, stages, kc, qcap);   // queue: qcap >= qflush - 1 + kChunk slots
@@ -689,6 +694,14 @@ __global__ void __launch_bounds__(kAP2Threads, 1)
     const float pf_k = 1.4426950408889634f / noise_scale;
     const bool pf_scale_ok = NOISE == 2 && noise_scale > 1e-20f && noise_scale < 1e20f && !no_prefilter;
     bool prefilter = pf_scale_ok;
+    float ubv = INFINITY;    // CONT: the previous pass's last entry of this row (idx -1: it ran out of columns)
+    int ubc = -1;
+    if (CONT && after_val != nullptr && row_ok) {
+      ubc = __ldg(after_idx + (size_t)lrow * after_ld);
+      ubv = ubc < 0 ? -INFINITY : __ldg(after_val + (size_t)lrow * after_ld);
+    }
+    auto after_bound = [&](float yy, int j) { return !CONT || yy < ubv || (yy == ubv && j > ubc); };
+    const int ld = CONT ? out_ld : kc;
     auto flush = [&](unsigned need) {
       __syncwarp();
       while (need) {
@@ -762,7 +775,7 @@ __global__ void __launch_bounds__(kAP2Threads, 1)
                 for (int c = 0; c < kChunk; ++c) {
                   if (pass & (1u << (kChunk - 1 - c))) {
                     const float yy = y[c] + gumbel_from_bits(xb[c], noise_scale);
-                    if (jbase + c < n && yy > thr) {
+                    if (jbase + c < n && yy > thr && after_bound(yy, jbase + c)) {
                       qv[qn * kBM + row_t] = yy;
                       qi[qn * kBM + row_t] = jbase + c;
                       ++qn;
@@ -787,7 +800,7 @@ __global__ void __launch_bounds__(kAP2Threads, 1)
               }
               y[c] = yy;
               if (NOISE == 3 && j < n) zsum += __expf(yy * inv_temp);   // evaluation branch only
-              pass |= (j < n && yy > thr) ? (1u << c) : 0u;
+              pass |= (j < n && yy > thr && after_bound(yy, j)) ? (1u << c) : 0u;
             }
             if (pass) {
 #pragma unroll
@@ -835,8 +848,8 @@ __global__ void __launch_bounds__(kAP2Threads, 1)
         }
         for (int r = lane; r < kc; r += kWarp) {
           const int32_t id = idxs[r * kBM + rt];
-          out_idx[(size_t)lr * kc + r] = id;
-          out_val[(size_t)lr * kc + r] = id < 0 ? 0.f : vals[r * kBM + rt];
+          out_idx[(size_t)lr * ld + r] = id;
+          out_val[(size_t)lr * ld + r] = id < 0 ? 0.f : vals[r * kBM + rt];
         }
       }
       if (out_rowsum != nullptr && row_ok) out_rowsum[lrow] = zsum + zpart[row_t];
@@ -910,6 +923,23 @@ __global__ void __launch_bounds__(kMergeWarps* kWarp)
 // ------------------------------------------------------------------------------------------------
 constexpr int kPairWarps = 8;
 
+// V features per lane: 4 (one float4, d % 4 == 0) or 1 (any d)
+template <int V>
+__device__ __forceinline__ void ldg_v(float (&r)[V], const float* p) {
+  if constexpr (V == 4) {
+    const float4 f = ldg4(p);
+    r[0] = f.x; r[1] = f.y; r[2] = f.z; r[3] = f.w;
+  } else {
+    r[0] = __ldg(p);
+  }
+}
+template <int V>
+__device__ __forceinline__ void red_add_v(float* p, const float (&r)[V], float sign) {
+  if constexpr (V == 4) red_add4(p, make_float4(sign * r[0], sign * r[1], sign * r[2], sign * r[3]));
+  else atomicAdd(p, sign * r[0]);
+}
+
+template <int V>
 __global__ void __launch_bounds__(kPairWarps* kWarp)
     allpairs_pair_grad_kernel(const float* __restrict__ z, int n, int d, int L, int row_begin, int row_count,
                               const int32_t* __restrict__ idx, const float* __restrict__ gy, int kc,
@@ -922,11 +952,13 @@ __global__ void __launch_bounds__(kPairWarps* kWarp)
     const int i = row_begin + lr;
     if (i >= n) continue;
     const float* zi = z + (size_t)i * d;
-    for (int c0 = 0; c0 < d; c0 += 4 * L) {   // feature chunks of 4*L columns (one float4 per lane)
-      const int c = c0 + 4 * lg;
+    for (int c0 = 0; c0 < d; c0 += V * L) {   // feature chunks of V*L columns
+      const int c = c0 + V * lg;
       const bool cok = c < d;
-      const float4 a = cok ? ldg4(zi + c) : make_float4(0.f, 0.f, 0.f, 0.f);
-      float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+      float a[V], acc[V];
+#pragma unroll
+      for (int v = 0; v < V; ++v) a[v] = acc[v] = 0.f;
+      if (cok) ldg_v<V>(a, zi + c);
       for (int r0 = 0; r0 < kc; r0 += G) {
         const int r = r0 + grp;
         const int j = (r < kc) ? __ldg(idx + (size_t)lr * kc + r) : -1;
@@ -934,27 +966,34 @@ __global__ void __launch_bounds__(kPairWarps* kWarp)
         // full squared distance needs every chunk: recompute it over all of d (d is small)
         float dist2 = 0.f;
         if (j >= 0)
-          for (int cc = 4 * lg; cc < d; cc += 4 * L) {
-            const float4 p = ldg4(zi + cc), qv = ldg4(z + (size_t)j * d + cc);
-            const float dx = p.x - qv.x, dy_ = p.y - qv.y, dz_ = p.z - qv.z, dw = p.w - qv.w;
-            dist2 += dx * dx + dy_ * dy_ + dz_ * dz_ + dw * dw;
+          for (int cc = V * lg; cc < d; cc += V * L) {
+            float p[V], qv[V];
+            ldg_v<V>(p, zi + cc);
+            ldg_v<V>(qv, z + (size_t)j * d + cc);
+            float s = (p[0] - qv[0]) * (p[0] - qv[0]);
+#pragma unroll
+            for (int v = 1; v < V; ++v) s += (p[v] - qv[v]) * (p[v] - qv[v]);
+            dist2 += s;
           }
         dist2 = group_sum(dist2, L);
         const float dist = sqrtf(dist2);
         if (c0 == 0 && lg == 0) dt_acc += -dist * g_up;
         const float g = (dist > 0.f) ? (-t * g_up / dist) : 0.f;
         if (j >= 0 && cok && g != 0.f) {
-          const float4 b = ldg4(z + (size_t)j * d + c);
-          const float4 dd = make_float4(g * (a.x - b.x), g * (a.y - b.y), g * (a.z - b.z), g * (a.w - b.w));
-          acc.x += dd.x; acc.y += dd.y; acc.z += dd.z; acc.w += dd.w;
-          red_add4(dz + (size_t)j * d + c, make_float4(-dd.x, -dd.y, -dd.z, -dd.w));
+          float b[V];
+          ldg_v<V>(b, z + (size_t)j * d + c);
+#pragma unroll
+          for (int v = 0; v < V; ++v) {
+            b[v] = g * (a[v] - b[v]);
+            acc[v] += b[v];
+          }
+          red_add_v<V>(dz + (size_t)j * d + c, b, -1.f);
         }
       }
-      for (int o = L; o < kWarp; o <<= 1) {
-        acc.x += __shfl_xor_sync(0xffffffffu, acc.x, o); acc.y += __shfl_xor_sync(0xffffffffu, acc.y, o);
-        acc.z += __shfl_xor_sync(0xffffffffu, acc.z, o); acc.w += __shfl_xor_sync(0xffffffffu, acc.w, o);
-      }
-      if (grp == 0 && cok) red_add4(dz + (size_t)i * d + c, acc);
+      for (int o = L; o < kWarp; o <<= 1)
+#pragma unroll
+        for (int v = 0; v < V; ++v) acc[v] += __shfl_xor_sync(0xffffffffu, acc[v], o);
+      if (grp == 0 && cok) red_add_v<V>(dz + (size_t)i * d + c, acc, 1.f);
     }
   }
   dt_acc = warp_sum(dt_acc);
@@ -1059,7 +1098,6 @@ extern "C" int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d
   // slots (flushed whenever anything is pending) to keep two stages + both groups' lists under 227 KB
   const bool big = (kb == 4 && precision == 3);
   const int qcap = big ? kChunk : kQCap, qflush = big ? 1 : kQFlush;
-  if (after_val != nullptr && big) return DGGB_ERR_K_OVERFLOW;   // continuation passes run on the v1 kernel only
   if (kc <= 32 && (want_v2 || big) && after_val == nullptr) {
     int st2 = 4;
     AP2Smem L2 = ap2_smem_layout(kb, precision, st2, kc, qcap);
@@ -1086,7 +1124,7 @@ extern "C" int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d
     allpairs_topk2_kernel<KB_, SP_, NM_><<<grid2d, kAP2Threads, smem2, st>>>(                                     \
         tm_hi, tm_lo, hi, lo, npad, dpad, nrm, n, row_begin, row_count, t, noise, (long long)noise_ld,            \
         (unsigned long long)seed, noise_scale, kc, st2, qcap, qflush, out_idx, out_val, inv_temp, out_rowsum,     \
-        no_pf, tpp, part_idx, part_val);                                                                          \
+        no_pf, tpp, part_idx, part_val, kc, nullptr, nullptr, 0);                                                 \
   } while (0)
 #define DGGB_AP2_LAUNCH(KB_, SP_)                                                                                 \
   do {                                                                                                            \
@@ -1113,6 +1151,42 @@ extern "C" int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d
       }
       return launch_status();
     }
+  }
+  // the same tile shape beyond one plain v2 call (kc 33..64, continuation passes): v1 has no instantiation for it, so
+  // the continuation instantiation of v2 runs it, kc > 32 as two passes whose second admits only what sorts after
+  // the first pass's last entry of the row (ranks 32..kc-1)
+  if (big) {
+    const int no_pf = getenv("DGGB_AP_NO_PREFILTER") ? 1 : 0;
+    auto cont_pass = [&](int kcp, int32_t* oi, float* ov, const float* av, const int32_t* ai, int ald,
+                         float* rs) -> int {
+      int st2 = 4;
+      AP2Smem L2 = ap2_smem_layout(kb, precision, st2, kcp, qcap);
+      while (st2 > 2 && L2.total + 1024 > 227 * 1024) L2 = ap2_smem_layout(kb, precision, --st2, kcp, qcap);
+      if (L2.total + 1024 > 227 * 1024) return DGGB_ERR_BAD_SHAPE;
+      const size_t smem2 = L2.total + 1024;
+      const dim3 grid2d((row_count + kBM - 1) / kBM, 1);
+      const int tpp = (n + kBN - 1) / kBN;
+#define DGGB_AP2C_LAUNCH1(NM_)                                                                                    \
+  do {                                                                                                            \
+    cudaError_t e = cudaFuncSetAttribute(allpairs_topk2_kernel<4, 3, NM_, true>,                                  \
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);                \
+    if (e != cudaSuccess) return cuda_status(e);                                                                  \
+    allpairs_topk2_kernel<4, 3, NM_, true><<<grid2d, kAP2Threads, smem2, st>>>(                                   \
+        tm_hi, tm_lo, hi, lo, npad, dpad, nrm, n, row_begin, row_count, t, noise, (long long)noise_ld,            \
+        (unsigned long long)seed, noise_scale, kcp, st2, qcap, qflush, oi, ov, inv_temp, rs, no_pf, tpp, nullptr, \
+        nullptr, kc, av, ai, ald);                                                                                \
+  } while (0)
+      if (nmode2 == 0) DGGB_AP2C_LAUNCH1(0);
+      else if (nmode2 == 1) DGGB_AP2C_LAUNCH1(1);
+      else if (nmode2 == 2) DGGB_AP2C_LAUNCH1(2);
+      else DGGB_AP2C_LAUNCH1(3);
+#undef DGGB_AP2C_LAUNCH1
+      return launch_status();
+    };
+    if (kc <= 32) return cont_pass(kc, out_idx, out_val, after_val, after_idx, 1, out_rowsum);
+    rc = cont_pass(32, out_idx, out_val, after_val, after_idx, 1, out_rowsum);
+    if (rc != DGGB_OK) return rc;
+    return cont_pass(kc - 32, out_idx + 32, out_val + 32, out_val + 31, out_idx + 31, kc, nullptr);
   }
   int stages = 4;
   APSmem L = ap_smem_layout(kb, precision, stages, kc);
@@ -1156,10 +1230,13 @@ extern "C" int dggb_allpairs_pair_bwd(const float* z, int32_t n, int32_t d, int3
                                       const int32_t* idx, const float* gy, int32_t kc, const float* t, float* dz,
                                       float* dt, void* stream) {
   if (!z || !idx || !gy || !t || !dz || !dt || n <= 0 || d <= 0 || row_count < 0 || kc <= 0) return DGGB_ERR_BAD_ARG;
-  if (d % 4 != 0) return DGGB_ERR_BAD_SHAPE;
   if (row_count == 0) return DGGB_OK;
-  const int L = pow2_floor32(d / 4);
-  allpairs_pair_grad_kernel<<<rows_grid(row_count, kPairWarps, 8), kPairWarps * kWarp, 0, as_stream(stream)>>>(
-      z, n, d, L, row_begin, row_count, idx, gy, kc, t, dz, dt);
+  const dim3 grid(rows_grid(row_count, kPairWarps, 8));
+  if (d % 4 == 0)   // one float4 per lane
+    allpairs_pair_grad_kernel<4><<<grid, kPairWarps * kWarp, 0, as_stream(stream)>>>(
+        z, n, d, pow2_floor32(d / 4), row_begin, row_count, idx, gy, kc, t, dz, dt);
+  else              // rows of z are not 16-byte aligned: one float per lane
+    allpairs_pair_grad_kernel<1><<<grid, kPairWarps * kWarp, 0, as_stream(stream)>>>(
+        z, n, d, pow2_floor32(d), row_begin, row_count, idx, gy, kc, t, dz, dt);
   return launch_status();
 }
