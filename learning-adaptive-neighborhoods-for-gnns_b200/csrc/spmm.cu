@@ -1107,7 +1107,8 @@ extern "C" int dggb_spmm_gemm_fwd(const int32_t* rowptr, const int32_t* col, con
     return launch_status();
   };
   const int Q = fout <= 32 ? 1 : (fout <= 64 ? 2 : 4);
-  static const bool no_row = getenv("DGGB_SPMM_GEMM_NO_ROW") != nullptr;      // A/B: entry-parallel kernel on small graphs
+  // A/B: entry-parallel kernel on small graphs; read per call, so that one process can run both paths
+  const bool no_row = getenv("DGGB_SPMM_GEMM_NO_ROW") != nullptr;
   if (rb == 1 && !no_row)
     return Q == 1 ? go(spmm_gemm_fwd_row_kernel<1>) : (Q == 2 ? go(spmm_gemm_fwd_row_kernel<2>) : go(spmm_gemm_fwd_row_kernel<4>));
 #define DGGB_SG_Q(T_, R_) (Q == 1 ? go(spmm_gemm_fwd_kernel<T_, 1, R_>) : (Q == 2 ? go(spmm_gemm_fwd_kernel<T_, 2, R_>) : go(spmm_gemm_fwd_kernel<T_, 4, R_>)))

@@ -156,7 +156,10 @@ class _Spmm(torch.autograd.Function):
         # (Pubmed shape, F = 64, inside a CUDA graph: forward 9.7 us incl. the zero fill vs 15.2 warp-per-row,
         # backward 7.7 vs 21.7 us)
         ctx.edge = (not _NO_EDGE_SPMM) and f % 4 == 0 and f <= 512 and graph.nnz > 0 and graph.nnz <= 64 * n
-        if ctx.edge:
+        if graph.nnz == 0:
+            # no entries: Y = 0.  The entry points reject the NULL col / val pointers of empty tensors
+            y = torch.zeros(n, f, dtype=torch.float32, device=x.device)
+        elif ctx.edge:
             y = torch.zeros(n, f, dtype=torch.float32, device=x.device)
             check(lib().dggb_spmm_edge_fwd(p(graph.rowptr), p(graph.erow), p(graph.col), p(vals), i32(n),
                                            i64(graph.nnz), p(x), i32(f), p(row_scale), p(y), stream()), "spmm_edge_fwd")
@@ -178,7 +181,7 @@ class _Spmm(torch.autograd.Function):
         if ctx.edge:
             check(lib().dggb_spmm_edge_bwd(p(g.erow), p(g.col), p(vals), i64(g.nnz), p(x), i32(x.shape[1]),
                                            p(row_scale), p(_f32c(gy)), p(dval), p(dx), stream()), "spmm_edge_bwd")
-        else:
+        elif g.nnz > 0:                                                      # no entries: dx stays 0, dval is empty
             check(lib().dggb_spmm_csr_bwd(p(g.rowptr), p(g.col), p(vals), i32(g.n), p(x), i32(x.shape[1]),
                                           p(row_scale), p(_f32c(gy)), p(dval), p(dx), stream()), "spmm_csr_bwd")
         return dval, dx, None, None
