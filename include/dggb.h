@@ -453,6 +453,57 @@ int dggb_induced_subgraph_fill(const int32_t* rowptr, const int32_t* col, const 
                                const int32_t* relabel, const int32_t* sub_rowptr, int32_t* sub_col, int32_t* sub_eid,
                                void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * k-hop neighbour sampling on the device: what torch_geometric.loader.NeighborLoader (torch_sparse / pyg-lib
+ * neighbor_sample, third-party, not in the reference tree) does for train_pubmed.py:370-375.  Parity with PyG is
+ * unpinned: the RNG stream differs and so does the within-target order of Floyd's picks; tests/neighbor_ref.py
+ * restates the contract below as a sequential loop and the kernels match it bit for bit.
+ *
+ * The parent graph is in CSC form, colptr[n+1] / row[nnz]: the entries of target v are its in-neighbours (sources u
+ * of the edges u -> v) sorted by source; multi-edges stay separate entries.  Hop l (0-based, l < 255) has frontier F_l
+ * and fanout k_l: F_0 = the seeds, F_{l+1} = the nodes first discovered in hop l, in discovery order.  For frontier
+ * slot t (position in F_l) with target v and d = deg_in(v):
+ *   - d == 0 or k == 0: nothing;
+ *   - k < 0, or replace == 0 and k >= d: all d entries in ascending position;
+ *   - replace == 1: k draws, draw i emits position floor(x_i * d / 2^32), in draw order;
+ *   - otherwise Floyd's algorithm (as torch_sparse): for i = 0..k-1, j = d - k + i, r = floor(x_i * (j+1) / 2^32);
+ *     add r to the set, or j if r is already in it; the k positions are emitted in ascending order.
+ *   x_i = 32-bit lane (i & 3) of Philox4x32-7(counter = (t, (l << 24) | (i >> 2)), key = seed) (csrc/philox.cuh).
+ *   k <= 1024 (larger: DGGB_ERR_BAD_SHAPE); k = -1 means "all".
+ * Emissions of a hop are ordered by slot, then by the per-target order above.  A source not yet in n_id gets the next
+ * local id at its first emission (torch_sparse's sequential rule); every emission is one edge (local(u), local(v)).
+ *
+ * Workspace: local[n] (local id or -1) and claim[n] (INT_MAX when idle), filled once by the caller; a batch leaves
+ * them as it found them once dggb_neighbor_reset has run over its n_id.  Per batch:
+ *   dggb_neighbor_seed: local[seeds[t]] = t; *status = 1 if a seed is out of range or repeated, else 0.
+ * Per hop (frontier[m], the local id of slot t is frontier_base + t):
+ *   dggb_neighbor_count: counts[m] int64 emissions per slot; the caller scans them (int64, inclusive) into offsets
+ *     and reads the total T, which must be <= 2^31 - 1;
+ *   dggb_neighbor_sample: out_pos[T] (CSC positions), out_dst[T] (target local ids), and claim[u] = the smallest
+ *     emission index of every source u with local[u] < 0;
+ *   dggb_neighbor_flag: flags[T] = 1 at the first emission of each new source; the caller scans them (int32,
+ *     inclusive) into scan and reads the number of new nodes;
+ *   dggb_neighbor_assign: new_nodes[id] = u and local[u] = base + id, id = scan[e] - 1 at each flagged emission.
+ * Once the last hop is assigned:
+ *   dggb_neighbor_edges: edge_index[2, count] int64 = (local source, dst) of every emission (hops concatenated);
+ *   dggb_neighbor_reset: local[u] = -1, claim[u] = INT_MAX for the nodes[count] of the batch.
+ * ---------------------------------------------------------------------------------- */
+int dggb_neighbor_seed(const int32_t* seeds, int32_t num_seeds, int32_t n, int32_t* local, int64_t* status,
+                       void* stream);
+int dggb_neighbor_count(const int32_t* colptr, int32_t n, const int32_t* frontier, int32_t m, int32_t k,
+                        int32_t replace, int64_t* counts, void* stream);
+int dggb_neighbor_sample(const int32_t* colptr, const int32_t* row, const int32_t* frontier, int32_t m, int32_t k,
+                         int32_t replace, int32_t hop, uint64_t seed, int32_t frontier_base, const int64_t* offsets,
+                         const int32_t* local, int32_t* claim, int32_t* out_pos, int32_t* out_dst, void* stream);
+int dggb_neighbor_flag(const int32_t* row, const int32_t* pos, int32_t count, const int32_t* local,
+                       const int32_t* claim, int32_t* flags, void* stream);
+int dggb_neighbor_assign(const int32_t* row, const int32_t* pos, int32_t count, const int32_t* flags,
+                         const int32_t* scan, int32_t base, int32_t* local, int32_t* new_nodes, void* stream);
+int dggb_neighbor_edges(const int32_t* row, const int32_t* pos, const int32_t* dst, int64_t count,
+                        const int32_t* local, int64_t* edge_index, void* stream);
+int dggb_neighbor_reset(const int32_t* nodes, int32_t count, int32_t n, int32_t* local, int32_t* claim,
+                        void* stream);
+
 #ifdef __cplusplus
 }
 #endif

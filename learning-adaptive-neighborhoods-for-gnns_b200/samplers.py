@@ -1,4 +1,4 @@
-"""Device-side sub-graph sampler for the large-graph drivers (SURVEY 8f rank 2).
+"""Device-side sub-graph samplers for the mini-batch drivers (SURVEY 8f rank 2).
 
 ``train_large_graphs.py:402-413`` / ``train_reddit.py:400-411`` build their mini-batches with
 ``torch_geometric.loader.GraphSAINTRandomWalkSampler(data, batch_size=, walk_length=, num_steps=, sample_coverage=,
@@ -16,8 +16,17 @@ start nodes ``torch.randint(0, N, (batch_size,))`` from the global CPU generator
 of the scripts seeds), uniform neighbour choice per step, walkers on a node without out-edges stay, the batch is the
 sub-graph induced by the sorted unique visited nodes with all parent edges between them in row-major order, and the
 normalisation statistics are visit counts over pre-sampled batches (``edge_norm = node_count[row] / edge_count``
-clamped to 1e4, ``node_norm = num_samples / node_count / N``).  The Cluster / Neighbor loaders the scripts can also
-select are not provided.
+clamped to 1e4, ``node_norm = num_samples / node_count / N``).
+
+``train_pubmed.py:370-375`` feeds its mini-batches from ``torch_geometric.loader.NeighborLoader(data,
+num_neighbors=[50, 50], ...)``.  ``NeighborLoader`` here follows the PyG 2.x constructor and batch surface for
+homogeneous graphs (``n_id``, ``e_id``, ``batch_size``, ``num_sampled_nodes``, ``num_sampled_edges``, node / edge
+attributes sliced by them) and samples on the GPU with ``neighbor_sample`` over ``dggb_neighbor_*``
+(csrc/neighbor.cu): a without-replacement draw per target (Floyd's algorithm, as torch_sparse) or k draws with
+replacement, then the de-duplication and relabelling of the sampled nodes in torch_sparse's sequential order.  Samples
+are NOT PyG's samples for the same seed: the RNG stream differs (Philox keyed on the batch seed, the hop, the frontier
+slot and the draw) and so does the within-target order of Floyd's picks (ascending here).  Parity is pinned only
+against the restatement in tests/neighbor_ref.py.  ``ClusterLoader`` is not provided (it needs a METIS partitioner).
 """
 from __future__ import annotations
 
@@ -52,6 +61,21 @@ def _data_items(data):
     if keys is None:
         keys = [k for k in vars(data) if not k.startswith("_")]
     return [(k, getattr(data, k)) for k in keys]
+
+
+def _split_attrs(data, n, e, dev):
+    """-> (node attributes [n, ...] on dev, edge attributes [e, ...] on dev, everything else), by leading size."""
+    node_attrs, edge_attrs, other = {}, {}, {}
+    for k, v in _data_items(data):
+        if k in ("edge_index", "num_nodes"):
+            continue
+        if torch.is_tensor(v) and v.dim() > 0 and v.shape[0] == n:
+            node_attrs[k] = v.to(dev)
+        elif torch.is_tensor(v) and v.dim() > 0 and v.shape[0] == e:
+            edge_attrs[k] = v.to(dev)
+        else:
+            other[k] = v
+    return node_attrs, edge_attrs, other
 
 
 def induced_subgraph(graph: CSRGraph, nodes: torch.Tensor):
@@ -106,16 +130,7 @@ class GraphSAINTRandomWalkSampler:
         key = ei[0] * self.N + ei[1]
         self.perm = torch.argsort(key, stable=True)
         self.graph = CSRGraph.from_indices(ei[:, self.perm].contiguous(), self.N)
-        self._node_attrs, self._edge_attrs, self._other = {}, {}, {}
-        for k, v in _data_items(data):
-            if k in ("edge_index", "num_nodes"):
-                continue
-            if torch.is_tensor(v) and v.dim() > 0 and v.shape[0] == self.N:
-                self._node_attrs[k] = v.to(dev)
-            elif torch.is_tensor(v) and v.dim() > 0 and v.shape[0] == self.E:
-                self._edge_attrs[k] = v.to(dev)
-            else:
-                self._other[k] = v
+        self._node_attrs, self._edge_attrs, self._other = _split_attrs(data, self.N, self.E, dev)
         self.node_norm = self.edge_norm = None
         if self.sample_coverage > 0:
             self.node_norm, self.edge_norm = self._compute_norm()
@@ -169,3 +184,193 @@ class GraphSAINTRandomWalkSampler:
     def __iter__(self):
         for _ in range(self.num_steps):
             yield self._collate(*self._sample())
+
+
+# ------------------------------------------------------------------------------------------------ neighbour sampling
+_MAX_FANOUT, _MAX_HOPS, _INT32_MAX = 1024, 255, 2 ** 31 - 1
+
+
+def _neighbor_workspace(csc: CSRGraph):
+    """(local int32 [N] = -1, claim int32 [N] = INT32_MAX), allocated once per graph; every call puts back the entries
+    it touched."""
+    ws = csc.aux.get("neighbor_ws")
+    if ws is None:
+        dev = csc.col.device
+        ws = (torch.full((csc.n,), -1, dtype=torch.int32, device=dev),
+              torch.full((csc.n,), _INT32_MAX, dtype=torch.int32, device=dev))
+        csc.aux["neighbor_ws"] = ws
+    return ws
+
+
+def neighbor_sample(csc: CSRGraph, seeds: torch.Tensor, num_neighbors, seed: int, replace: bool = False):
+    """k-hop neighbour sampling on the device (the contract of ``dggb_neighbor_*`` in include/dggb.h).
+
+    ``csc``: the parent graph over in-neighbours, as a CSRGraph whose ``rowptr`` is the CSC colptr and whose ``col``
+    holds the sources: the entries of target v are the u of the edges u -> v, sorted by u.  ``seeds``: unique int32
+    node ids on the device.  ``num_neighbors``: fanout per hop, -1 for every in-neighbour, at most 1024.  ``seed``:
+    the 64-bit Philox key.
+
+    Returns ``(n_id, edge_index, pos, num_sampled_nodes, num_sampled_edges)``: ``n_id`` int32 [M] with the seeds first
+    and then each hop's new nodes in discovery order; ``edge_index`` int64 [2, E] of local ids (row 0 the source, row 1
+    the target); ``pos`` int32 [E], the CSC position of every sampled entry; the two per-hop count lists.
+
+    Two device->host reads per hop with a non-empty frontier: the hop's emission total (it sizes the outputs) and its
+    number of new nodes (it sizes the next frontier).  The workspace (2 x int32 [N]) is allocated once per graph in
+    ``csc.aux``; each call resets only the entries of the nodes it sampled, so calls that share a graph must run on
+    one stream.
+    """
+    assert seeds.is_cuda and seeds.dtype == torch.int32 and seeds.dim() == 1
+    num_neighbors = [int(k) for k in num_neighbors]
+    if len(num_neighbors) > _MAX_HOPS or any(k < -1 or k > _MAX_FANOUT for k in num_neighbors):
+        raise ValueError(f"num_neighbors: at most {_MAX_HOPS} hops of -1 ... {_MAX_FANOUT} neighbours each")
+    L = lib()
+    local, claim = _neighbor_workspace(csc)
+    dev, b, n = seeds.device, int(seeds.numel()), csc.n
+    colptr, row = csc.rowptr, csc.col
+    nodes, pos_parts, dst_parts = [seeds], [], []
+    num_nodes, num_edges = [b], []
+    try:
+        head = torch.empty(b + 1, dtype=torch.int64, device=dev)      # hop 0's offsets, then the seed status
+        # an empty tensor has no data pointer, and the entry points reject NULL: calls with nothing to do are skipped
+        if b > 0:
+            check(L.dggb_neighbor_seed(p(seeds), i32(b), i32(n), p(local), p(head[b:]), stream()), "neighbor_seed")
+        if b > 0 and not num_neighbors and int(head[b]):
+            raise ValueError("seeds must be unique node ids in [0, N)")
+        frontier = seeds
+        for hop, k in enumerate(num_neighbors):
+            m = int(frontier.numel())
+            if m == 0:
+                num_nodes.append(0)
+                num_edges.append(0)
+                continue
+            counts = torch.empty(m, dtype=torch.int64, device=dev)
+            check(L.dggb_neighbor_count(p(colptr), i32(n), p(frontier), i32(m), i32(k), i32(int(replace)), p(counts),
+                                        stream()), "neighbor_count")
+            offsets = head if hop == 0 else torch.empty(m, dtype=torch.int64, device=dev)
+            torch.cumsum(counts, 0, out=offsets[:m])
+            if hop == 0:
+                total, bad = offsets[m - 1:].tolist()                  # one read: the total and the seed status
+                if bad:
+                    raise ValueError("seeds must be unique node ids in [0, N)")
+            else:
+                total = int(offsets[m - 1])
+            if total > _INT32_MAX:
+                raise ValueError(f"hop {hop} would sample {total} edges (more than 2^31 - 1): lower num_neighbors")
+            num_edges.append(total)
+            if total == 0:
+                num_nodes.append(0)
+                frontier = frontier[:0]
+                continue
+            out_pos = torch.empty(total, dtype=torch.int32, device=dev)
+            out_dst = torch.empty(total, dtype=torch.int32, device=dev)
+            check(L.dggb_neighbor_sample(p(colptr), p(row), p(frontier), i32(m), i32(k), i32(int(replace)), i32(hop),
+                                         int(seed) & 0xFFFFFFFFFFFFFFFF, i32(sum(num_nodes[:-1])), p(offsets),
+                                         p(local), p(claim), p(out_pos), p(out_dst), stream()), "neighbor_sample")
+            flags = torch.empty(total, dtype=torch.int32, device=dev)
+            check(L.dggb_neighbor_flag(p(row), p(out_pos), i32(total), p(local), p(claim), p(flags), stream()),
+                  "neighbor_flag")
+            scan = torch.cumsum(flags, 0, dtype=torch.int32)
+            new = int(scan[-1])
+            new_nodes = torch.empty(new, dtype=torch.int32, device=dev)
+            if new > 0:
+                check(L.dggb_neighbor_assign(p(row), p(out_pos), i32(total), p(flags), p(scan), i32(sum(num_nodes)),
+                                             p(local), p(new_nodes), stream()), "neighbor_assign")
+            nodes.append(new_nodes)
+            pos_parts.append(out_pos)
+            dst_parts.append(out_dst)
+            num_nodes.append(new)
+            frontier = new_nodes
+        n_id = torch.cat(nodes)
+        pos = torch.cat(pos_parts) if pos_parts else torch.empty(0, dtype=torch.int32, device=dev)
+        dst = torch.cat(dst_parts) if dst_parts else pos
+        e = int(pos.numel())
+        edge_index = torch.empty(2, e, dtype=torch.int64, device=dev)
+        if e > 0:
+            check(L.dggb_neighbor_edges(p(row), p(pos), p(dst), i64(e), p(local), p(edge_index), stream()),
+                  "neighbor_edges")
+        if b > 0:
+            check(L.dggb_neighbor_reset(p(n_id), i32(n_id.numel()), i32(n), p(local), p(claim), stream()),
+                  "neighbor_reset")
+    except BaseException:
+        csc.aux.pop("neighbor_ws", None)       # part of a batch is still registered: the next call starts afresh
+        raise
+    return n_id, edge_index, pos, num_nodes, num_edges
+
+
+class NeighborLoader:
+    """``for batch in loader``: PyG 2.x ``torch_geometric.loader.NeighborLoader`` over one homogeneous graph, sampled
+    on the GPU by ``neighbor_sample``.
+
+    Batches of ``batch_size`` input nodes come from a ``torch.utils.data.DataLoader`` over the input indices, so the
+    ``shuffle`` order follows the global CPU generator as in PyG; each batch then draws its 62-bit sampling seed from
+    the same generator.  Worker arguments (``num_workers``, ``persistent_workers``, ...) are accepted and ignored.
+    A batch is a ``SubgraphBatch`` with the node attributes of the parent sliced by ``n_id`` and its edge attributes by
+    ``e_id`` (the caller's edge ids), ``edge_index`` (local ids, row 0 the source), ``n_id``, ``e_id``,
+    ``batch_size``, ``num_sampled_nodes`` and ``num_sampled_edges``; its first ``batch_size`` nodes are the batch's
+    input nodes, in input order.
+    """
+
+    def __init__(self, data, num_neighbors, input_nodes=None, replace=False, directed=True, batch_size=1,
+                 shuffle=False, drop_last=False, device=None, **kwargs):
+        if not directed:
+            raise NotImplementedError("NeighborLoader(directed=False) is not provided")
+        if kwargs.get("disjoint"):
+            raise NotImplementedError("NeighborLoader(disjoint=True) is not provided")
+        if kwargs.get("time_attr") is not None:
+            raise NotImplementedError("temporal sampling (time_attr) is not provided")
+        if (isinstance(num_neighbors, dict) or isinstance(input_nodes, (tuple, str))
+                or hasattr(data, "node_types") or hasattr(data, "edge_types")):
+            raise NotImplementedError("heterogeneous graphs are not provided")
+        assert data.edge_index is not None
+        self.num_neighbors = [int(k) for k in num_neighbors]
+        self.replace = bool(replace)
+        dev = torch.device(device) if device is not None else (
+            data.edge_index.device if data.edge_index.is_cuda else torch.device("cuda"))
+        self.device = dev
+        self.N = int(getattr(data, "num_nodes", None) or data.x.shape[0])
+        if input_nodes is None:
+            nodes = torch.arange(self.N)
+        else:
+            nodes = torch.as_tensor(input_nodes).cpu()
+            if nodes.dtype == torch.bool:
+                if nodes.shape != (self.N,):
+                    raise ValueError(f"input_nodes mask has shape {tuple(nodes.shape)}, expected ({self.N},)")
+                nodes = nodes.nonzero().view(-1)
+            nodes = nodes.long().view(-1)
+        if nodes.numel() and (int(nodes.min()) < 0 or int(nodes.max()) >= self.N):
+            raise ValueError(f"input_nodes holds ids outside [0, {self.N})")
+        if torch.unique(nodes).numel() != nodes.numel():
+            raise ValueError("input_nodes holds repeated nodes")
+        self.input_nodes = nodes.to(torch.int32)
+        ei = data.edge_index.to(dev)
+        self.E = int(ei.shape[1])
+        # parent adjacency in CSC order (targets, then sources); perm maps a CSC position to the caller's edge id
+        self.perm = torch.argsort(ei[1] * self.N + ei[0], stable=True)
+        self.csc = CSRGraph.from_indices(ei.flip(0)[:, self.perm].contiguous(), self.N)
+        self._node_attrs, self._edge_attrs, self._other = _split_attrs(data, self.N, self.E, dev)
+        self._loader = torch.utils.data.DataLoader(range(int(nodes.numel())), batch_size=batch_size, shuffle=shuffle,
+                                                   drop_last=drop_last, collate_fn=self._collate)
+
+    def __len__(self):
+        return len(self._loader)
+
+    def __iter__(self):
+        return iter(self._loader)
+
+    def _collate(self, index):
+        seeds = self.input_nodes[torch.as_tensor(index, dtype=torch.long)].to(self.device)
+        seed = int(torch.randint(0, 2 ** 62, (1,), dtype=torch.long))          # global CPU generator
+        n_id, edge_index, pos, num_nodes, num_edges = neighbor_sample(self.csc, seeds, self.num_neighbors, seed,
+                                                                      self.replace)
+        nl = n_id.long()
+        e_id = self.perm[pos.long()]
+        batch = SubgraphBatch(num_nodes=int(nl.numel()), edge_index=edge_index, n_id=nl, e_id=e_id,
+                              batch_size=int(seeds.numel()), num_sampled_nodes=num_nodes,
+                              num_sampled_edges=num_edges)
+        for k, v in self._node_attrs.items():
+            setattr(batch, k, v[nl])
+        for k, v in self._edge_attrs.items():
+            setattr(batch, k, v[e_id])
+        for k, v in self._other.items():
+            setattr(batch, k, v)
+        return batch
