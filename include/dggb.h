@@ -81,7 +81,8 @@ int dggb_add_self_loops_fill(const int32_t* rowptr, const int32_t* col, const fl
  * warp-per-row rank pass.  The dense N x N scatter, the N-long row sort and the un-sort scatter of the reference
  * are not performed: off-support entries are exact zeros that sort last, so the rank
  * inside the row's own edges is the rank in the dense row.
- * Requires H % 4 == 0.
+ * Requires H % 4 == 0.  nnz == 0 is allowed (erow, col, R, rank, out, and g_out in the backward, may then be
+ * NULL): every row gets s = 0 and k = LeakyReLU(deg_b), and the backward adds nothing.
  * ---------------------------------------------------------------------------------- */
 int dggb_dgg_edge_fwd(const int32_t* rowptr, const int32_t* erow /* [E] row of each entry */,
                       const int32_t* col, int32_t n, int32_t nnz, int32_t h,
@@ -109,8 +110,11 @@ int dggb_dgg_edge_bwd(const int32_t* rowptr, const int32_t* erow, const int32_t*
 /* Single-launch variants of the two calls above for graphs whose longest row has at most 512 entries
  * (max_row_nnz: the caller's cached max over rows of rowptr[i+1]-rowptr[i]; Cora / Citeseer / Pubmed qualify).
  * A block owns the rows that start inside its slice of the entry range, keeps their scores (fwd) / ds (bwd) in
- * shared memory and runs both phases back to back.  Same arguments, same results bit for bit.
- * Return DGGB_ERR_UNSUPPORTED when max_row_nnz > 512 or nnz == 0: call the two-launch entry point instead. */
+ * shared memory and runs both phases back to back.  Same arguments.  R and rank are the two-launch results bit for
+ * bit; s, k, out and the gradients differ from them by the summation order of the row sums (and of the atomics).
+ * Return DGGB_ERR_UNSUPPORTED when max_row_nnz > 512 or nnz == 0: call the two-launch entry point instead.
+ * DGGB_FUSED_EPB (read per call; values below 1 are ignored) sets the smallest number of entries per block, and
+ * DGGB_FUSED_V1 selects the first-generation kernels (see csrc/dgg_edge.cu). */
 int dggb_dgg_edge_fwd_fused(const int32_t* rowptr, const int32_t* erow, const int32_t* col, int32_t n,
                             int32_t nnz, int32_t max_row_nnz, int32_t h, const float* y, const float* be,
                             const float* deg_w, const float* deg_b, const float* ablation_noise,

@@ -452,7 +452,8 @@ __global__ void __launch_bounds__(kEdgeWarps* kWarp)
 // epb + max_deg entries.  fwd: edge-parallel scores into shared memory -> __syncthreads -> warp-per-row rank from
 // shared memory.  bwd: warp-per-row dk/ds into shared memory -> __syncthreads -> edge-parallel gradients.
 // At Pubmed shape the two-launch path is pure latency (2 x ~12 us for 0.4 MB of edge data); this is one wave of
-// blocks with ~4 dependent memory round trips.  Results are bit-identical to the two-launch kernels.
+// blocks with ~4 dependent memory round trips.  R and rank are bit-identical to the two-launch kernels; s, k and
+// out differ from them by the summation order of the row sums.
 // ------------------------------------------------------------------------------------------------
 constexpr int kFusedMaxDeg = 512;
 constexpr int kFusedThreads = 256;
@@ -1041,8 +1042,11 @@ __global__ void __launch_bounds__(kFusedThreads, DGGB_BWD2_MIN_BLOCKS)
 }
 
 // grid of the fused kernels: at most one wave (blocks_per_sm from the occupancy calculator), >= 128 edges per block (measured 256 / 128 / 64: forward 16.8 / 14.1 / 14.1 us at Pubmed shape; DGGB_FUSED_EPB overrides)
+// The override is read per call, so that one process can run several grids; values below 1 are ignored.
 static void fused_grid(int nnz, int blocks_per_sm, int* blocks, int* epb) {
-  static const int min_epb = getenv("DGGB_FUSED_EPB") ? atoi(getenv("DGGB_FUSED_EPB")) : 128;
+  const char* env = getenv("DGGB_FUSED_EPB");
+  const int env_epb = env ? atoi(env) : 0;
+  const int min_epb = env_epb >= 1 ? env_epb : 128;
   long long b = ((long long)nnz + min_epb - 1) / min_epb;
   const long long cap = (long long)kNumSMs * (blocks_per_sm < 1 ? 1 : blocks_per_sm);
   if (b > cap) b = cap;
@@ -1051,11 +1055,17 @@ static void fused_grid(int nnz, int blocks_per_sm, int* blocks, int* epb) {
   *blocks = (nnz + *epb - 1) / *epb;
 }
 
-// DGGB_FUSED_V1=1: first-generation fused kernels (A/B measurements)
-static bool fused_v1() {
-  static const bool v1 = getenv("DGGB_FUSED_V1") != nullptr;
-  return v1;
+// Without an opt-in a block gets at most 48 KB of shared memory, static and dynamic together: the largest score
+// windows (12 288 floats in the forward, 2 x 6 144 in the backward) plus the kernels' static arrays exceed it.  The
+// opt-in is only requested for large windows, so the small graphs' launches make no extra call.
+template <typename K>
+static int allow_dynamic_smem(K kern, size_t smem) {
+  if (smem <= 40 * 1024) return DGGB_OK;
+  return cuda_status(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 }
+
+// DGGB_FUSED_V1=1: first-generation fused kernels (A/B measurements); read per call, like DGGB_FUSED_EPB
+static bool fused_v1() { return getenv("DGGB_FUSED_V1") != nullptr; }
 
 static int edges_grid(long long nnz, int blocks_per_sm = 8) {
   long long need = (nnz + kEdgeWarps * kWarp - 1) / (kEdgeWarps * kWarp);
@@ -1072,8 +1082,9 @@ extern "C" int dggb_dgg_edge_fwd(const int32_t* rowptr, const int32_t* erow, con
                                  int32_t nnz, int32_t h, const float* y, const float* be, const float* deg_w,
                                  const float* deg_b, const float* ablation_noise, int32_t hard_k, float* R,
                                  int32_t* rank, float* s, float* k, float* out, int32_t* long_ws, void* stream) {
-  if (!rowptr || !erow || !col || !y || !be || !deg_w || !deg_b || !R || !rank || !s || !k || !out || n < 0 ||
-      nnz < 0 || h <= 0)
+  // the per-entry arrays may be NULL when there are no entries (an empty tensor has no data pointer)
+  if (!rowptr || !y || !be || !deg_w || !deg_b || !s || !k || n < 0 || nnz < 0 || h <= 0 ||
+      (nnz > 0 && (!erow || !col || !R || !rank || !out)))
     return DGGB_ERR_BAD_ARG;
   if (h % 4 != 0 || h > 512) return DGGB_ERR_BAD_SHAPE;
   if (n == 0) return DGGB_OK;
@@ -1101,8 +1112,8 @@ extern "C" int dggb_dgg_edge_bwd(const int32_t* rowptr, const int32_t* erow, con
                                  const float* deg_b, const float* ablation_noise, int32_t hard_k, const float* R,
                                  const int32_t* rank, const float* s, const float* k, const float* g_out,
                                  float* ds_ws, float* dy, float* dbe, float* ddeg, void* stream) {
-  if (!rowptr || !erow || !col || !y || !be || !deg_w || !deg_b || !R || !rank || !s || !k || !g_out || !ds_ws ||
-      !dy || !dbe || !ddeg || n < 0 || nnz < 0 || h <= 0)
+  if (!rowptr || !y || !be || !deg_w || !deg_b || !s || !k || !ds_ws || !dy || !dbe || !ddeg || n < 0 || nnz < 0 ||
+      h <= 0 || (nnz > 0 && (!erow || !col || !R || !rank || !g_out)))
     return DGGB_ERR_BAD_ARG;
   if (h % 4 != 0 || h > 512) return DGGB_ERR_BAD_SHAPE;
   if (n == 0 || nnz == 0) return DGGB_OK;
@@ -1167,6 +1178,8 @@ extern "C" int dggb_dgg_edge_fwd_fused(const int32_t* rowptr, const int32_t* ero
     // shared-memory score window: entries beyond it (bounded-degree graphs with > ~7 M entries make epb large)
     // are re-read from global memory by the rank phase (the `idx < cap` / `in_s` guards of the kernel)
     const int cap = min(epb + max_row_nnz, 12288);
+    const int st = allow_dynamic_smem(kern, (size_t)cap * sizeof(float));
+    if (st != DGGB_OK) return st;
     launch_pdl(kern, dim3(blocks), dim3(kFusedThreads), (size_t)cap * sizeof(float), as_stream(stream), rowptr, erow,
                col, n, nnz, h, L, epb, cap, y, be, ablation_noise, deg_w, deg_b, hard_k, R, rank, s, k, out, zero_ws,
                (long long)zero_count);
@@ -1229,6 +1242,8 @@ extern "C" int dggb_dgg_edge_bwd_fused(const int32_t* rowptr, const int32_t* ero
     const int cap = epb + max_row_nnz;
     *fits = cap <= 6144;
     if (!*fits) return (int)DGGB_OK;
+    const int st = allow_dynamic_smem(kern, (size_t)cap * 2 * sizeof(float));
+    if (st != DGGB_OK) return st;
     launch_pdl(kern, dim3(blocks), dim3(kFusedThreads), (size_t)cap * 2 * sizeof(float), as_stream(stream), rowptr,
                erow, col, n, nnz, h, L, epb, cap, y, be, ablation_noise, hard_k, R, rank, s, k, g_out, deg_w, deg_b,
                ds_ws, dy, dbe, ddeg);

@@ -97,7 +97,9 @@ class _DGGEdge(torch.autograd.Function):
         dy = zbuf[:n * h].view(n, h)
         small = zbuf[n * h:]
         dbe, ddeg, ds_ws = small[:h], small[h:h + 2], small[h + 4:]
-        if ctx.fused_mx > 0:
+        if g.nnz == 0:
+            pass                             # no entries: every gradient is 0, nothing to launch
+        elif ctx.fused_mx > 0:
             check(lib().dggb_dgg_edge_bwd_fused(p(g.rowptr), p(g.erow), p(g.col), i32(n), i32(g.nnz), i32(ctx.fused_mx),
                                                 i32(h), p(y), p(be), p(deg_w), p(deg_b), p(noise), i32(ctx.hard_k),
                                                 p(R), p(rank), p(s), p(k), p(_f32c(g_out)), p(ds_ws), p(dy), p(dbe),
@@ -468,8 +470,9 @@ class _RowFirstK(torch.autograd.Function):
         score, k = _f32c(score), _f32c(k).reshape(-1)
         rank = torch.empty(graph.nnz, dtype=torch.int32, device=score.device)
         out = torch.empty_like(score)
-        check(lib().dggb_row_firstk_fwd(p(graph.rowptr), i32(graph.n), p(score), p(k), i32(mode), p(rank), p(out),
-                                        p(_long_ws(graph)), stream()), "row_firstk_fwd")
+        if graph.nnz > 0:   # no entries: empty outputs (the entry point rejects the NULL pointers of empty tensors)
+            check(lib().dggb_row_firstk_fwd(p(graph.rowptr), i32(graph.n), p(score), p(k), i32(mode), p(rank), p(out),
+                                            p(_long_ws(graph)), stream()), "row_firstk_fwd")
         ctx.graph, ctx.mode = graph, mode
         ctx.save_for_backward(score, k, rank)
         ctx.mark_non_differentiable(rank)
@@ -480,6 +483,8 @@ class _RowFirstK(torch.autograd.Function):
         score, k, rank = ctx.saved_tensors
         gr = ctx.graph
         dscore = torch.empty_like(score)
+        if gr.nnz == 0:
+            return (dscore if ctx.mode == 0 else None), torch.zeros_like(k), None, None
         dk = torch.empty_like(k)
         check(lib().dggb_row_firstk_bwd(p(gr.rowptr), i32(gr.n), p(score), p(k), i32(ctx.mode), p(rank), p(_f32c(g)),
                                         p(dscore), p(dk), stream()), "row_firstk_bwd")

@@ -34,7 +34,9 @@ class CSRGraph:
         """int32 [nnz] row index of every entry (built once per structure)."""
         if self._erow is None:
             self._erow = torch.empty(self.nnz, dtype=torch.int32, device=self.col.device)
-            check(lib().dggb_csr_expand_rows(p(self.rowptr), i32(self.n), p(self._erow), stream()), "csr_expand_rows")
+            if self.nnz > 0:   # no entries: nothing to write (and an empty tensor has no data pointer to pass)
+                check(lib().dggb_csr_expand_rows(p(self.rowptr), i32(self.n), p(self._erow), stream()),
+                      "csr_expand_rows")
         return self._erow
 
     @property
