@@ -508,6 +508,77 @@ int dggb_neighbor_edges(const int32_t* row, const int32_t* pos, const int32_t* d
 int dggb_neighbor_reset(const int32_t* nodes, int32_t count, int32_t n, int32_t* local, int32_t* claim,
                         void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * Deterministic multilevel k-way graph partitioning on the device: what METIS does for torch_geometric.loader.ClusterData
+ * (train_large_graphs.py:402-421; third-party, host cores).  The partitions are NOT METIS's: parity is unpinned;
+ * tests/cluster_ref.py restates every phase below and the driver of dgg_b200.samplers.partition, and the kernels match
+ * it bit for bit.  Integer arithmetic only; atomics compute only sums and minima, so no result depends on the order in
+ * which blocks or atomics run.
+ *
+ * A level is a symmetric CSR rowptr[n+1] / col[nnz] (rows sorted, no self loops, no duplicates) with entry weights
+ * ewt[nnz] >= 1 and node weights vw[n] >= 1.  A labelling lab[n] assigns every node a label (a cluster while
+ * coarsening, a part while refining) in [0, nlabels).  h(x) = MurmurHash3's fmix32.  NONE = INT64_MAX.
+ *   dggb_partition_weights: lw[L] = sum of vw over the nodes labelled L; anchor[L] = the smallest such node, or
+ *     0x7f7f7f7f (anchor may be NULL).
+ *   dggb_partition_propose: key[n].  Each active node v finds the adjacent label L != lab[v] with
+ *     lw[L] + vw[v] <= limit that has the largest (conn(L), h(L)), conn(L) = summed ewt of v's entries into L, and
+ *     gain = conn(L) - conn(lab[v]).  mode 0 (cluster): active when (h(v) & 1) == parity; proposes L when gain > 0.
+ *     mode 1 (refine): as 0, and v != anchor[lab[v]] (a part is never left empty).  mode 3 (unload): as 1, and
+ *     lw[lab[v]] > limit; proposes L whatever the gain.  A proposal is key = L << 32 | (uint32)(2^31 - 1 - gain), no
+ *     proposal NONE.  mode 2 (evict): every v != anchor[lab[v]] with lw[lab[v]] > limit (parity ignored) gets
+ *     key = lab[v] << 32 | (uint32)(2^31 - 1 - gain), conn(L) = 0 when there is no L.  anchor may be NULL in mode 0.
+ *   The caller sorts the keys stably (node id breaks ties) into keys[n] / order[n] (int64).
+ *   dggb_partition_admit: cum[n] = inclusive int64 scan of vw[order].  Each run of equal target t = key >> 32 is
+ *     admitted in order while lw[t] (start-of-round weight) + the run's weight up to and including the node <= limit:
+ *     lab[order[i]] = t.
+ *   dggb_partition_rebalance (unit node weights): for the evict keys of mode 2 with limit = cap, the first
+ *     lw[p] - cap nodes of each over-full part p (least gain lost first) take the free places cap - lw[q] of the parts
+ *     below cap in part order: ex_prefix[k] = exclusive scan of max(lw - cap, 0), room_cum[k] = inclusive scan of
+ *     max(cap - lw, 0), both int64.
+ *   dggb_partition_contract_keys: keys[nnz] = cluster[row] * nc + cluster[col] of every entry, NONE inside a cluster.
+ *     The caller sorts them (any sort: idx[nnz] = the source entry of each sorted key).
+ *   dggb_partition_contract_heads: heads[nnz] int32 = 1 at the first of each run of equal sorted keys (not NONE); the
+ *     caller scans them (int32, inclusive) into scan and reads cnnz = scan[nnz-1].
+ *   dggb_partition_contract_fill: coarse entry j = scan - 1 of a run: crow[j] (int64), ccol[j], cwt[j] = summed ewt[idx].
+ *   dggb_partition_bfs: order[n], pos[n] (position in order) of a level-synchronous BFS: a frontier node's unvisited
+ *     neighbours follow it ordered by (parent position, id); a new search starts from the smallest unvisited id.
+ *     claim[n] is scratch.  One block: meant for the coarsest level.
+ *   dggb_partition_chunk: part[order[i]] = min(k - 1, prefix[i] * k / total), prefix = exclusive int64 scan of
+ *     vw[order], total = its sum.
+ *   dggb_partition_project: out[v] = map[idx[v]].
+ * ClusterLoader batches over the parent CSR permuted so that every part is a contiguous id range:
+ *   dggb_cluster_batch_count / _fill: drawn part b covers parent ids [start[b], end[b]) and local ids from base[b];
+ *     rows node_idx[m] are the drawn parts' ids in draw order.  count: counts[m] kept entries per row (columns inside
+ *     a drawn part); the caller scans them into sub_rowptr[m + 1].  fill: each row's kept entries in ascending local
+ *     id, i.e. one ascending run per drawn part in draw order: sub_col (local id), sub_eid (position in the parent CSR).
+ * ---------------------------------------------------------------------------------- */
+int dggb_partition_weights(const int32_t* lab, const int32_t* vw, int32_t n, int32_t nlabels, int32_t* lw,
+                           int32_t* anchor, void* stream);
+int dggb_partition_propose(const int32_t* rowptr, const int32_t* col, const int32_t* ewt, const int32_t* vw,
+                           const int32_t* lab, int32_t n, const int32_t* lw, const int32_t* anchor, int32_t limit,
+                           int32_t parity, int32_t mode, int64_t* key, void* stream);
+int dggb_partition_admit(const int64_t* keys, const int64_t* order, const int64_t* cum, int32_t n, const int32_t* lw,
+                         int32_t limit, int32_t* lab, void* stream);
+int dggb_partition_rebalance(const int64_t* keys, const int64_t* order, int32_t n, const int32_t* lw,
+                             const int64_t* ex_prefix, const int64_t* room_cum, int32_t k, int32_t cap, int32_t* part,
+                             void* stream);
+int dggb_partition_contract_keys(const int32_t* rowptr, const int32_t* col, int32_t n, const int32_t* cluster,
+                                 int32_t nc, int64_t* keys, void* stream);
+int dggb_partition_contract_heads(const int64_t* keys, int64_t nnz, int32_t* heads, void* stream);
+int dggb_partition_contract_fill(const int64_t* keys, const int64_t* idx, const int32_t* ewt, int64_t nnz,
+                                 const int32_t* scan, int32_t nc, int32_t cnnz, int64_t* crow, int32_t* ccol,
+                                 int32_t* cwt, void* stream);
+int dggb_partition_bfs(const int32_t* rowptr, const int32_t* col, int32_t n, int32_t* order, int32_t* pos,
+                       int32_t* claim, void* stream);
+int dggb_partition_chunk(const int32_t* order, const int64_t* prefix, int32_t n, int64_t total, int32_t k,
+                         int32_t* part, void* stream);
+int dggb_partition_project(const int32_t* map, const int32_t* idx, int32_t n, int32_t* out, void* stream);
+int dggb_cluster_batch_count(const int32_t* rowptr, const int32_t* col, const int32_t* start, const int32_t* end,
+                             int32_t num_drawn, const int32_t* node_idx, int32_t m, int32_t* counts, void* stream);
+int dggb_cluster_batch_fill(const int32_t* rowptr, const int32_t* col, const int32_t* start, const int32_t* end,
+                            const int32_t* base, int32_t num_drawn, const int32_t* node_idx, int32_t m,
+                            const int32_t* sub_rowptr, int32_t* sub_col, int32_t* sub_eid, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -26,7 +26,14 @@ attributes sliced by them) and samples on the GPU with ``neighbor_sample`` over 
 replacement, then the de-duplication and relabelling of the sampled nodes in torch_sparse's sequential order.  Samples
 are NOT PyG's samples for the same seed: the RNG stream differs (Philox keyed on the batch seed, the hop, the frontier
 slot and the draw) and so does the within-target order of Floyd's picks (ascending here).  Parity is pinned only
-against the restatement in tests/neighbor_ref.py.  ``ClusterLoader`` is not provided (it needs a METIS partitioner).
+against the restatement in tests/neighbor_ref.py.
+
+The Cluster-GCN branch of ``train_large_graphs.py`` uses ``torch_geometric.loader.ClusterData`` (METIS on host cores
+through torch_sparse) and ``ClusterLoader``.  ``ClusterData`` / ``ClusterLoader`` here follow the PyG 2.1 surface and
+partition on the GPU with ``partition`` over ``dggb_partition_*`` (csrc/partition.cu): a deterministic multilevel k-way
+partitioner (size-constrained label-propagation coarsening, a BFS-order split of the coarsest graph, label-propagation
+refinement and an exact rebalance), every part non-empty and at most ``ceil(1.03 N / num_parts)`` nodes.  The parts
+are NOT METIS's: parity is pinned only against the restatement in tests/cluster_ref.py.
 """
 from __future__ import annotations
 
@@ -374,3 +381,330 @@ class NeighborLoader:
         for k, v in self._other.items():
             setattr(batch, k, v)
         return batch
+
+
+# ------------------------------------------------------------------------------------------------ graph partitioning
+# Constants of the multilevel driver (tests/cluster_ref.py restates it with the same values).
+_CMAX_DIV = 1             # cluster weight limit while coarsening: N // (_CMAX_DIV * num_parts), at least 1
+_STOP_PER_PART = 2        # coarsen while the graph has more than _STOP_PER_PART * num_parts nodes
+_MIN_SHRINK = (19, 20)    # ... and a level keeps fewer than 19/20 of its nodes
+_MAX_LEVELS = 32
+_LP_ROUNDS = 5            # label-propagation rounds per coarsening level (two sub-rounds each)
+_REFINE_ROUNDS = 4        # refinement rounds per level (two sub-rounds each)
+_REBALANCE_ROUNDS = 2     # rounds per level that move nodes out of over-full parts into adjacent parts
+
+
+class _Level:
+    """One level of the hierarchy: symmetric int32 CSR with int32 entry weights ewt and node weights vw."""
+
+    def __init__(self, n, rowptr, col, ewt, vw):
+        self.n, self.rowptr, self.vw = n, rowptr, vw
+        self.nnz = int(col.numel())
+        # an empty tensor has no data pointer and the entry points reject NULL: a one-entry stand-in (never read,
+        # every row is empty)
+        self.col = col if self.nnz else torch.zeros(1, dtype=torch.int32, device=rowptr.device)
+        self.ewt = ewt if self.nnz else torch.ones(1, dtype=torch.int32, device=rowptr.device)
+
+
+def _cap(n, k):
+    return (103 * n + 100 * k - 1) // (100 * k)
+
+
+def _symmetrize(edge_index, n, dev):
+    """-> _Level 0: both directions of every edge, self loops dropped, duplicates merged, unit weights."""
+    ei = edge_index.to(dev, torch.int64)
+    u, v = torch.cat([ei[0], ei[1]]), torch.cat([ei[1], ei[0]])
+    keep = u != v
+    key = torch.unique(u[keep] * n + v[keep])                   # sorted
+    g = CSRGraph.from_indices(torch.stack([key // n, key % n]), n)
+    ones = torch.ones(n, dtype=torch.int32, device=dev)
+    return _Level(n, g.rowptr, g.col, torch.ones(g.nnz, dtype=torch.int32, device=dev), ones)
+
+
+def _weights(lab, vw, nlabels, with_anchor=True):
+    dev = lab.device
+    lw = torch.empty(nlabels, dtype=torch.int32, device=dev)
+    anchor = torch.empty(nlabels, dtype=torch.int32, device=dev) if with_anchor else None
+    check(lib().dggb_partition_weights(p(lab), p(vw), i32(lab.numel()), i32(nlabels), p(lw), p(anchor), stream()),
+          "partition_weights")
+    return lw, anchor
+
+
+def _propose(g, lab, lw, anchor, limit, parity, mode):
+    key = torch.empty(g.n, dtype=torch.int64, device=lab.device)
+    check(lib().dggb_partition_propose(p(g.rowptr), p(g.col), p(g.ewt), p(g.vw), p(lab), i32(g.n), p(lw), p(anchor),
+                                       i32(limit), i32(parity), i32(mode), p(key), stream()), "partition_propose")
+    return torch.sort(key, stable=True)                          # ties: node id ascending
+
+
+def _lp_rounds(g, lab, nlabels, limit, rounds, mode):
+    for _ in range(rounds):
+        for parity in (0, 1):
+            lw, anchor = _weights(lab, g.vw, nlabels, with_anchor=mode != 0)
+            keys, order = _propose(g, lab, lw, anchor, limit, parity, mode)
+            cum = torch.cumsum(g.vw[order], 0, dtype=torch.int64)
+            check(lib().dggb_partition_admit(p(keys), p(order), p(cum), i32(g.n), p(lw), i32(limit), p(lab), stream()),
+                  "partition_admit")
+    return lab
+
+
+def _project(map_, idx):
+    out = torch.empty(idx.numel(), dtype=torch.int32, device=idx.device)
+    check(lib().dggb_partition_project(p(map_), p(idx), i32(idx.numel()), p(out), stream()), "partition_project")
+    return out
+
+
+def _contract(g, cluster, nc):
+    """-> the coarse _Level: one node per cluster, the entries between clusters merged with summed weights."""
+    L, dev = lib(), cluster.device
+    rowptr = torch.zeros(nc + 1, dtype=torch.int32, device=dev)
+    cvw = _weights(cluster, g.vw, nc, with_anchor=False)[0]
+    cnnz = 0
+    if g.nnz:
+        keys = torch.empty(g.nnz, dtype=torch.int64, device=dev)
+        check(L.dggb_partition_contract_keys(p(g.rowptr), p(g.col), i32(g.n), p(cluster), i32(nc), p(keys), stream()),
+              "partition_contract_keys")
+        keys, idx = torch.sort(keys)
+        heads = torch.empty(g.nnz, dtype=torch.int32, device=dev)
+        check(L.dggb_partition_contract_heads(p(keys), i64(g.nnz), p(heads), stream()), "partition_contract_heads")
+        scan = torch.cumsum(heads, 0, dtype=torch.int32)
+        cnnz = int(scan[-1])
+    ccol = torch.empty(cnnz, dtype=torch.int32, device=dev)
+    cwt = torch.empty(cnnz, dtype=torch.int32, device=dev)
+    if cnnz:
+        crow = torch.empty(cnnz, dtype=torch.int64, device=dev)
+        check(L.dggb_partition_contract_fill(p(keys), p(idx), p(g.ewt), i64(g.nnz), p(scan), i32(nc), i32(cnnz),
+                                             p(crow), p(ccol), p(cwt), stream()), "partition_contract_fill")
+        check(L.dggb_coo_rows_to_rowptr(p(crow), i64(cnnz), i32(nc), p(rowptr), stream()), "coo_rows_to_rowptr")
+    return _Level(nc, rowptr, ccol, cwt, cvw)
+
+
+def _initial(g, k):
+    """BFS order of the coarsest level cut into k chunks of equal weight."""
+    L, dev = lib(), g.rowptr.device
+    order = torch.empty(g.n, dtype=torch.int32, device=dev)
+    pos = torch.empty(g.n, dtype=torch.int32, device=dev)
+    claim = torch.empty(g.n, dtype=torch.int32, device=dev)
+    check(L.dggb_partition_bfs(p(g.rowptr), p(g.col), i32(g.n), p(order), p(pos), p(claim), stream()), "partition_bfs")
+    w = g.vw[order.long()].long()
+    prefix = torch.cumsum(w, 0) - w
+    total = int(prefix[-1] + w[-1])
+    part = torch.empty(g.n, dtype=torch.int32, device=dev)
+    check(L.dggb_partition_chunk(p(order), p(prefix), i32(g.n), i64(total), i32(k), p(part), stream()),
+          "partition_chunk")
+    return part
+
+
+def _refine(g, part, k, cap):
+    part = _lp_rounds(g, part, k, cap, _REBALANCE_ROUNDS, 3)
+    return _lp_rounds(g, part, k, cap, _REFINE_ROUNDS, 1)
+
+
+def _rebalance(g, part, k, cap):
+    """Finest level (unit weights): the over-full parts hand their least-loss nodes to the parts with room."""
+    lw, anchor = _weights(part, g.vw, k)
+    if int(lw.max()) <= cap:
+        return part
+    keys, order = _propose(g, part, lw, anchor, cap, 0, 2)
+    excess = (lw.long() - cap).clamp_(min=0)
+    ex_prefix = torch.cumsum(excess, 0) - excess
+    room_cum = torch.cumsum((cap - lw.long()).clamp_(min=0), 0)
+    check(lib().dggb_partition_rebalance(p(keys), p(order), i32(g.n), p(lw), p(ex_prefix), p(room_cum), i32(k),
+                                         i32(cap), p(part), stream()), "partition_rebalance")
+    return _refine(g, part, k, cap)
+
+
+def _partition_parts(edge_index, n, k, dev):
+    """-> (part int32 [n] on dev, number of coarse levels).  The phases and their order are the contract of
+    ``dggb_partition_*`` in include/dggb.h; tests/cluster_ref.py restates this driver."""
+    if k == 1:
+        return torch.zeros(n, dtype=torch.int32, device=dev), 0
+    cap = _cap(n, k)
+    cmax = max(1, n // (_CMAX_DIV * k))
+    g = _symmetrize(edge_index, n, dev)
+    levels = []
+    while g.n > _STOP_PER_PART * k and len(levels) < _MAX_LEVELS:
+        lab = _lp_rounds(g, torch.arange(g.n, dtype=torch.int32, device=dev), g.n, cmax, _LP_ROUNDS, 0)
+        used = _weights(lab, g.vw, g.n, with_anchor=False)[0] > 0
+        cid = torch.cumsum(used, 0, dtype=torch.int32) - 1
+        nc = int(cid[-1]) + 1
+        if nc * _MIN_SHRINK[1] > g.n * _MIN_SHRINK[0]:
+            break
+        cluster = _project(cid, lab)
+        levels.append((g, cluster))
+        g = _contract(g, cluster, nc)
+    part = _refine(g, _initial(g, k), k, cap)
+    for fine, cluster in reversed(levels):
+        g = fine
+        part = _refine(g, _project(part, cluster), k, cap)
+    return _rebalance(g, part, k, cap), len(levels)
+
+
+def _edge_input(graph_or_edge_index, num_nodes):
+    if isinstance(graph_or_edge_index, CSRGraph):
+        g = graph_or_edge_index
+        return g.coo_indices(), g.n
+    ei = torch.as_tensor(graph_or_edge_index)
+    if ei.dim() != 2 or ei.shape[0] != 2:
+        raise ValueError(f"edge_index must be [2, E], got {tuple(ei.shape)}")
+    ei = ei.long()
+    if num_nodes is None:
+        num_nodes = int(ei.max()) + 1 if ei.numel() else 0
+    if ei.numel() and (int(ei.min()) < 0 or int(ei.max()) >= num_nodes):
+        raise ValueError(f"edge_index holds ids outside [0, {num_nodes})")
+    return ei, int(num_nodes)
+
+
+def partition(graph_or_edge_index, num_parts, num_nodes=None, device=None):
+    """Deterministic multilevel k-way partition on the GPU -> (perm int64 [N], partptr int64 [num_parts + 1]).
+
+    The graph is taken undirected (both directions of every edge, self loops dropped, duplicate pairs merged, unit
+    node and edge weights), as METIS is given it by torch_sparse.  Every part is non-empty and holds at most
+    ``ceil(1.03 N / num_parts)`` nodes; ``perm`` lists the nodes by (part, id) -- the stable form of torch_sparse's
+    ``cluster.sort()`` -- and part i is ``perm[partptr[i]:partptr[i+1]]``.  ``num_parts == 1`` is the identity.
+    The partitions are not METIS's; the same graph and ``num_parts`` give the same result on every run.
+    ``graph_or_edge_index``: a CSRGraph or an int [2, E] edge list (``num_nodes`` defaults to its largest id + 1).
+    """
+    ei, n = _edge_input(graph_or_edge_index, num_nodes)
+    k = int(num_parts)
+    if n < 1:
+        raise ValueError("partition: the graph has no nodes")
+    if not 1 <= k <= n:
+        raise ValueError(f"num_parts must be in [1, {n}], got {k}")
+    dev = torch.device(device) if device is not None else (ei.device if ei.is_cuda else torch.device("cuda"))
+    part, _ = _partition_parts(ei, n, k, dev)
+    perm = torch.argsort(part, stable=True)
+    partptr = torch.zeros(k + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(torch.bincount(part, minlength=k), 0, out=partptr[1:])
+    return perm, partptr
+
+
+def _structure_hash(edge_index, n):
+    import hashlib
+
+    h = hashlib.sha256(f"{n}:{int(edge_index.shape[1])}:".encode())
+    h.update(edge_index.detach().to("cpu", torch.int64).contiguous().numpy().tobytes())
+    return h.hexdigest()
+
+
+class ClusterData:
+    """PyG 2.1 ``torch_geometric.loader.ClusterData`` over one homogeneous graph, partitioned on the GPU by
+    ``partition`` (not METIS: the parts differ from PyG's, see the module docstring).
+
+    ``perm`` / ``partptr`` (int64, on the device): part i holds the permuted nodes ``partptr[i] ... partptr[i+1]-1``,
+    i.e. the original nodes ``perm[partptr[i]:partptr[i+1]]``.  ``data`` holds the node attributes permuted by
+    ``perm``, the edge attributes in the order of the permuted CSR (``data._csr``; ``data.e_id`` maps each CSR entry
+    to the caller's edge id; duplicate edges stay separate entries, in edge-id order) and ``edge_index`` of the permuted
+    graph.  ``recursive`` is accepted and changes nothing: PyG selects METIS's recursive bisection with it, and this
+    partitioner has one (direct k-way) scheme.  With ``save_dir`` the partition is cached in
+    ``save_dir/dggb_partition_{num_parts}.pt`` together with a hash of the edge structure; a file written for another
+    graph is recomputed and overwritten.  ``log`` prints one line when the partition is computed.
+    """
+
+    def __init__(self, data, num_parts, recursive=False, save_dir=None, log=True, device=None):
+        import os
+
+        assert data.edge_index is not None
+        dev = torch.device(device) if device is not None else (
+            data.edge_index.device if data.edge_index.is_cuda else torch.device("cuda"))
+        self.device, self.num_parts, self.recursive = dev, int(num_parts), bool(recursive)
+        n = int(getattr(data, "num_nodes", None) or data.x.shape[0])
+        ei = data.edge_index.to(dev).long()
+        self.N, self.E = n, int(ei.shape[1])
+        perm = partptr = None
+        path = os.path.join(save_dir, f"dggb_partition_{self.num_parts}.pt") if save_dir else None
+        digest = _structure_hash(ei, n) if path else None
+        if path and os.path.isfile(path):
+            saved = torch.load(path, map_location="cpu")
+            if isinstance(saved, dict) and saved.get("structure") == digest and saved.get("num_parts") == num_parts:
+                perm, partptr = saved["perm"].to(dev), saved["partptr"].to(dev)
+        if perm is None:
+            perm, partptr = partition(ei, self.num_parts, num_nodes=n, device=dev)
+            if log:
+                print(f"ClusterData: {n} nodes in {self.num_parts} parts (device partitioner)")
+            if path:
+                os.makedirs(save_dir, exist_ok=True)
+                torch.save(dict(structure=digest, num_parts=self.num_parts, perm=perm.cpu(), partptr=partptr.cpu()),
+                           path)
+        self.perm, self.partptr = perm, partptr
+        self._partptr_host = partptr.cpu().tolist()
+        inv = torch.empty_like(perm)
+        inv[perm] = torch.arange(n, device=dev)
+        row, col = inv[ei[0]], inv[ei[1]]
+        self.e_id = torch.argsort(row * n + col, stable=True)          # permuted CSR position -> caller's edge id
+        self.graph = CSRGraph.from_indices(torch.stack([row[self.e_id], col[self.e_id]]), n)
+        node_attrs, edge_attrs, other = _split_attrs(data, n, self.E, dev)
+        self._node_attrs = {k: v[perm] for k, v in node_attrs.items()}
+        self._edge_attrs = edge_attrs                                    # by the caller's edge id
+        self._other = other
+        self.data = SubgraphBatch(num_nodes=n, edge_index=self.graph.coo_indices(), e_id=self.e_id, **self._node_attrs,
+                                  **{k: v[self.e_id] for k, v in edge_attrs.items()}, **other)
+        self.data._csr = self.graph
+
+    def __len__(self):
+        return self.num_parts
+
+    def __getitem__(self, idx):
+        return self._batch([int(idx) % self.num_parts if int(idx) < 0 else int(idx)])
+
+    def _batch(self, parts):
+        """SubgraphBatch of the drawn parts, in draw order: PyG 2.1's narrow / index_select collate."""
+        if any(not 0 <= q < self.num_parts for q in parts):
+            raise IndexError(f"part index out of range [0, {self.num_parts})")
+        L, dev, pp = lib(), self.device, self._partptr_host
+        start = [pp[q] for q in parts]
+        end = [pp[q + 1] for q in parts]
+        base, m = [], 0
+        for s, e in zip(start, end):
+            base.append(m)
+            m += e - s
+        node_idx = torch.cat([torch.arange(s, e, dtype=torch.int32) for s, e in zip(start, end)]).to(dev)
+        meta = torch.tensor([start, end, base], dtype=torch.int32).to(dev)
+        nb = len(parts)
+        counts = torch.empty(m, dtype=torch.int32, device=dev)
+        check(L.dggb_cluster_batch_count(p(self.graph.rowptr), p(self.graph.col), p(meta[0]), p(meta[1]), i32(nb),
+                                         p(node_idx), i32(m), p(counts), stream()), "cluster_batch_count")
+        sub_rowptr = torch.zeros(m + 1, dtype=torch.int32, device=dev)
+        torch.cumsum(counts, 0, out=sub_rowptr[1:])
+        nnz = int(sub_rowptr[-1])
+        sub_col = torch.empty(nnz, dtype=torch.int32, device=dev)
+        sub_eid = torch.empty(nnz, dtype=torch.int32, device=dev)
+        if nnz:
+            check(L.dggb_cluster_batch_fill(p(self.graph.rowptr), p(self.graph.col), p(meta[0]), p(meta[1]),
+                                            p(meta[2]), i32(nb), p(node_idx), i32(m), p(sub_rowptr), p(sub_col),
+                                            p(sub_eid), stream()), "cluster_batch_fill")
+        sub = CSRGraph(m, sub_rowptr, sub_col)
+        nl = node_idx.long()
+        e_id = self.e_id[sub_eid.long()]
+        batch = SubgraphBatch(num_nodes=m, edge_index=sub.coo_indices())
+        for k, v in self._node_attrs.items():
+            setattr(batch, k, v[nl])
+        for k, v in self._edge_attrs.items():
+            setattr(batch, k, v[e_id])
+        for k, v in self._other.items():
+            setattr(batch, k, v)
+        batch._csr = sub           # consumers inside this package skip the edge list -> CSR conversion
+        return batch
+
+
+class ClusterLoader:
+    """PyG 2.1 ``torch_geometric.loader.ClusterLoader``: ``for batch in loader`` yields the sub-graph induced by
+    ``batch_size`` parts of a ``ClusterData`` at a time.  The parts come from a ``torch.utils.data.DataLoader`` over
+    the part indices, so the ``shuffle`` order follows the global CPU generator as in PyG.  A batch's nodes are the
+    drawn parts' nodes in draw order; its ``edge_index`` (local ids) is row-major with each row's columns ascending;
+    node attributes are sliced by those nodes and edge attributes by the caller's edge ids.  Worker arguments
+    (``num_workers``, ...) are accepted and ignored."""
+
+    def __init__(self, cluster_data, batch_size=1, shuffle=False, drop_last=False, **kwargs):
+        self.cluster_data = cluster_data
+        self._loader = torch.utils.data.DataLoader(range(len(cluster_data)), batch_size=batch_size, shuffle=shuffle,
+                                                   drop_last=drop_last, collate_fn=self._collate)
+
+    def __len__(self):
+        return len(self._loader)
+
+    def __iter__(self):
+        return iter(self._loader)
+
+    def _collate(self, index):
+        return self.cluster_data._batch([int(i) for i in index])
