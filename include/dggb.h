@@ -114,7 +114,31 @@ int dggb_dgg_edge_bwd(const int32_t* rowptr, const int32_t* erow, const int32_t*
  * bit; s, k, out and the gradients differ from them by the summation order of the row sums (and of the atomics).
  * Return DGGB_ERR_UNSUPPORTED when max_row_nnz > 512 or nnz == 0: call the two-launch entry point instead.
  * DGGB_FUSED_EPB (read per call; values below 1 are ignored) sets the smallest number of entries per block, and
- * DGGB_FUSED_V1 selects the first-generation kernels (see csrc/dgg_edge.cu). */
+ * DGGB_FUSED_V1 selects the first-generation kernels (see csrc/dgg_edge.cu).
+ *
+ * Training goes through the _mask pair.  The forward also stores what the backward would otherwise recompute from y:
+ *   branch_mask [E, ceil(H/32)] uint32: bit c % 32 of word c / 32 is set when pre_c = y_u - y_v + be > 0;
+ *   r1 [E]: the pre-noise sigmoid(z), written only when ablation_noise != NULL (then it is required with the mask).
+ * Both may be NULL (inference).  The backward reads them instead of y and be (8 B per entry at H = 64 instead of two
+ * 4 H-byte row gathers) and gives the gradients of the unmasked pair up to the order of the atomics.
+ *
+ * dggb_dgg_edge_bwd_fused, without a mask to read, runs the two-launch dggb_dgg_edge_bwd (same arguments, same
+ * accumulate-into contract, any dbe alignment); it stays for callers of this ABI. */
+int dggb_dgg_edge_fwd_fused_mask(const int32_t* rowptr, const int32_t* erow, const int32_t* col, int32_t n,
+                                 int32_t nnz, int32_t max_row_nnz, int32_t h, const float* y, const float* be,
+                                 const float* deg_w, const float* deg_b, const float* ablation_noise,
+                                 int32_t hard_k, float* R, int32_t* rank, float* s, float* k, float* out,
+                                 uint32_t* branch_mask /* [E, ceil(H/32)] out, or NULL */,
+                                 float* r1 /* [E] out when ablation_noise != NULL, or NULL */,
+                                 float* zero_ws, int64_t zero_count, void* stream);
+int dggb_dgg_edge_bwd_fused_mask(const int32_t* rowptr, const int32_t* erow, const int32_t* col, int32_t n,
+                                 int32_t nnz, int32_t max_row_nnz, int32_t h, const float* deg_w,
+                                 const float* deg_b, const float* ablation_noise, int32_t hard_k, const float* R,
+                                 const int32_t* rank, const float* s, const float* k,
+                                 const uint32_t* branch_mask /* [E, ceil(H/32)] from the forward */,
+                                 const float* r1 /* [E] from the forward when ablation_noise != NULL, or NULL */,
+                                 const float* g_out, float* ds_ws, float* dy, float* dbe, float* ddeg,
+                                 void* stream);
 int dggb_dgg_edge_fwd_fused(const int32_t* rowptr, const int32_t* erow, const int32_t* col, int32_t n,
                             int32_t nnz, int32_t max_row_nnz, int32_t h, const float* y, const float* be,
                             const float* deg_w, const float* deg_b, const float* ablation_noise,

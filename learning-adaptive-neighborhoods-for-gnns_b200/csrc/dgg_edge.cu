@@ -28,6 +28,78 @@ __device__ __forceinline__ float edge_partial(const RowSlice<T>& yu, const RowSl
   return z;
 }
 
+// Branch mask of an entry: [ceil(h / 32)] words, bit c % 32 of word c / 32 set when pre_c = y_u - y_v + be > 0, i.e.
+// when LeakyReLU'(pre_c) == 1.  The fused forward writes it so that the fused backward never gathers y again.
+// Lane lg's chunk t holds channels 4 (lg + L t) .. +3, all inside word (lg + L t) / 8: for L < 8 the L lanes of a group
+// share that word (= L t / 8, the same for every lane), for L >= 8 lanes 8j .. 8j + 7 do (a new word at every t).
+__device__ __forceinline__ int branch_word(int lg, int L, int t) { return (L < 8 ? L * t : lg + L * t) >> 3; }
+
+template <int T>
+struct BranchBits {
+  uint32_t w[T];
+};
+
+// edge_partial, and this lane's bits of every chunk t placed in word branch_word(lg, L, t) (chunks at c >= h: 0),
+// from one pass over pre_c.  z is summed exactly as edge_partial sums it.
+template <int T>
+__device__ __forceinline__ float edge_partial_bits(const RowSlice<T>& yu, const RowSlice<T>& yv, const RowSlice<T>& b,
+                                                   int lg, int L, BranchBits<T>& bb) {
+  float z = 0.f;
+#pragma unroll
+  for (int t = 0; t < T; ++t) {
+    const float px = yu.v[t].x - yv.v[t].x + b.v[t].x, py = yu.v[t].y - yv.v[t].y + b.v[t].y;
+    const float pz = yu.v[t].z - yv.v[t].z + b.v[t].z, pw = yu.v[t].w - yv.v[t].w + b.v[t].w;
+    z += leaky(px) + leaky(py) + leaky(pz) + leaky(pw);
+    const uint32_t nib = (uint32_t)(px > 0.f) | (uint32_t)(py > 0.f) << 1 | (uint32_t)(pz > 0.f) << 2 |
+                         (uint32_t)(pw > 0.f) << 3;
+    bb.w[t] = nib << ((4 * (lg + L * t)) & 31);
+  }
+  return z;
+}
+
+// The lanes of a word OR their bits and the word's first lane stores it.  Every lane of the warp calls this (the
+// word changes at the same t for all of them); `live` gates the stores.
+__device__ __forceinline__ void store_branch_word(uint32_t word, int wi, int h, int lg, int L, bool live,
+                                                  uint32_t* __restrict__ mrow) {
+  for (int o = 1; o < (L < 8 ? L : 8); o <<= 1) word |= __shfl_xor_sync(0xffffffffu, word, o);
+  if (live && (lg & 7) == 0 && 32 * wi < h) mrow[wi] = word;
+}
+
+template <int T>
+__device__ __forceinline__ void store_branch_mask(const BranchBits<T>& bb, int h, int lg, int L, bool live,
+                                                  uint32_t* __restrict__ mrow) {
+  uint32_t word = 0;
+  int wi = branch_word(lg, L, 0);
+#pragma unroll
+  for (int t = 0; t < T; ++t) {
+    const int wt = branch_word(lg, L, t);
+    if (wt != wi) {
+      store_branch_word(word, wi, h, lg, L, live, mrow);
+      word = 0;
+      wi = wt;
+    }
+    word |= bb.w[t];
+  }
+  store_branch_word(word, wi, h, lg, L, live, mrow);
+}
+
+// this lane's four bits of every chunk t (bit j: channel 4 (lg + L t) + j), 0 for dead slots and chunks at c >= h
+template <int T>
+__device__ __forceinline__ void load_branch_mask(uint32_t (&nib)[T], const uint32_t* __restrict__ mrow, int h, int lg,
+                                                 int L, bool live) {
+#pragma unroll
+  for (int t = 0; t < T; ++t) {
+    const int c = 4 * (lg + L * t);
+    nib[t] = (live && c < h) ? (__ldg(mrow + branch_word(lg, L, t)) >> (c & 31)) & 15u : 0u;
+  }
+}
+
+// d pre of one chunk: dz * LeakyReLU'(pre_c), the same products as dz * leaky_grad(pre_c)
+__device__ __forceinline__ float4 branch_scale(uint32_t nib, float dz) {
+  const float lo = dz * kLeaky;
+  return make_float4((nib & 1u) ? dz : lo, (nib & 2u) ? dz : lo, (nib & 4u) ? dz : lo, (nib & 8u) ? dz : lo);
+}
+
 __device__ __forceinline__ float first_k_plus_one(float r, float k) {
   // dgm.py:1801-1804: 1 - 0.5 * (1 + tanh(t - k)), then + 1.0
   const float fk = 1.f - 0.5f * (1.f + tanhf(r - k));
@@ -488,12 +560,14 @@ __global__ void __launch_bounds__(kFusedThreads)
                          const float* __restrict__ abl_noise, const float* __restrict__ deg_w,
                          const float* __restrict__ deg_b, int hard_k, float* R, int32_t* __restrict__ rank,
                          float* __restrict__ s_out, float* __restrict__ k_out, float* __restrict__ out,
-                         float* zero_ws, long long zero_count) {
+                         uint32_t* __restrict__ branch_mask, float* __restrict__ r1_out, float* zero_ws,
+                         long long zero_count) {
   pdl_trigger();
   if constexpr (LC > 0) {
     L = LC;
     h = 16 * LC;
   }
+  const int W = (h + 31) >> 5;           // branch-mask words per entry
   extern __shared__ float sR[];          // [cap] scores of this block's edge range
   __shared__ int rng[4];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -510,7 +584,7 @@ __global__ void __launch_bounds__(kFusedThreads)
     const int groups = (kFusedThreads / kWarp) * G;
     const int per = (nE + groups - 1) / groups;
     const int g0 = (warp * G + grp) * per;
-#pragma unroll 4
+#pragma unroll 1   // unrolled, the branch-mask bits push ptxas into small spills
     for (int it = 0; it < per; ++it) {
       const int idx = g0 + it;
       const bool valid = idx < nE;
@@ -519,10 +593,15 @@ __global__ void __launch_bounds__(kFusedThreads)
       RowSlice<T> yu, yv;
       load_slice<T>(yu, y + (size_t)u * h, h, lg, L, valid);
       load_slice<T>(yv, y + (size_t)v * h, h, lg, L, valid);
-      const float z = group_sum(edge_partial<T>(yu, yv, bias), L);
+      BranchBits<T> bb;   // formed whether or not it is stored: one code path keeps the register count of edge_partial
+      const float z = group_sum(edge_partial_bits<T>(yu, yv, bias, lg, L, bb), L);
+      if (branch_mask != nullptr) store_branch_mask<T>(bb, h, lg, L, valid, branch_mask + (size_t)e * W);
       if (valid && lg == 0) {
         float r = sigmoidf_(z);
-        if (abl_noise != nullptr) r = sigmoidf_(r + __ldg(abl_noise + e));  // dgm.py:1933-1935
+        if (abl_noise != nullptr) {
+          if (r1_out != nullptr) r1_out[e] = r;
+          r = sigmoidf_(r + __ldg(abl_noise + e));  // dgm.py:1933-1935
+        }
         R[e] = r;
         if (idx < cap) sR[idx] = r;
       }
@@ -602,7 +681,7 @@ template <int T, int LC>
 __global__ void __launch_bounds__(kFusedThreads)
     dgg_bwd_fused_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ erow,
                          const int32_t* __restrict__ col, int n, int nnz, int h, int L, int epb,
-                         const float* __restrict__ y, const float* __restrict__ be,
+                         const uint32_t* __restrict__ branch_mask, const float* __restrict__ r1_in,
                          const float* __restrict__ abl_noise, int hard_k, const float* __restrict__ R,
                          const int32_t* __restrict__ rank, const float* __restrict__ s_in,
                          const float* __restrict__ k_in, const float* __restrict__ g_out,
@@ -665,9 +744,9 @@ __global__ void __launch_bounds__(kFusedThreads)
     for (int wv = 0; wv < kFusedThreads / kWarp; ++wv) t += red[threadIdx.x][wv];
     if (t != 0.f) atomicAdd(ddeg + threadIdx.x, t);
   }
-  // ---- phase B: per edge, recompute z and scatter d pre ----
-  RowSlice<T> bias, dbe_acc, acc;
-  load_slice<T>(bias, be, h, lg, L);
+  // ---- phase B: per edge, d pre = dz LeakyReLU'(pre) from the forward's branch mask, scattered ----
+  const int W = (h + 31) >> 5;
+  RowSlice<T> dbe_acc, acc;
 #pragma unroll
   for (int t = 0; t < T; ++t) dbe_acc.v[t] = acc.v[t] = make_float4(0.f, 0.f, 0.f, 0.f);
   const int groups = (kFusedThreads / kWarp) * G;
@@ -694,12 +773,10 @@ __global__ void __launch_bounds__(kFusedThreads)
         dr *= r2 * (1.f - r2);  // through the second sigmoid
       }
     }
-    RowSlice<T> yu, yv;
-    load_slice<T>(yu, y + (size_t)u * h, h, lg, L);
-    load_slice<T>(yv, y + (size_t)v * h, h, lg, L);
-    const float z = group_sum(edge_partial<T>(yu, yv, bias), L);
-    const float r1s = sigmoidf_(z);
-    const float dz = valid ? dr * r1s * (1.f - r1s) : 0.f;
+    uint32_t nib[T];
+    load_branch_mask<T>(nib, branch_mask + (size_t)e * W, h, lg, L, valid);
+    const float r1e = __ldg(r1_in + e);
+    const float dz = valid ? dr * r1e * (1.f - r1e) : 0.f;
     if (valid && u != cur_u) {  // group-uniform branch: flush the finished source row
       if (cur_u >= 0) {
 #pragma unroll
@@ -714,11 +791,7 @@ __global__ void __launch_bounds__(kFusedThreads)
 #pragma unroll
     for (int t = 0; t < T; ++t) {
       const int c = 4 * (lg + L * t);
-      float4 d;
-      d.x = dz * leaky_grad(yu.v[t].x - yv.v[t].x + bias.v[t].x);
-      d.y = dz * leaky_grad(yu.v[t].y - yv.v[t].y + bias.v[t].y);
-      d.z = dz * leaky_grad(yu.v[t].z - yv.v[t].z + bias.v[t].z);
-      d.w = dz * leaky_grad(yu.v[t].w - yv.v[t].w + bias.v[t].w);
+      const float4 d = branch_scale(nib[t], dz);
       dbe_acc.v[t].x += d.x; dbe_acc.v[t].y += d.y; dbe_acc.v[t].z += d.z; dbe_acc.v[t].w += d.w;
       if (valid && u != v) {  // a self loop adds +d and -d to the same row: skip both (it still counts for dbe)
         acc.v[t].x += d.x; acc.v[t].y += d.y; acc.v[t].z += d.z; acc.v[t].w += d.w;
@@ -769,7 +842,9 @@ __global__ void __launch_bounds__(kFusedThreads)
 //     compare work is the same sum of deg^2, but spread evenly (a 171-entry row occupies 171 threads for 171
 //     iterations instead of one 8-lane group for 3 600);
 //   * backward: entry-parallel as well -- per-entry d out / d k terms into shared memory, each entry's thread sums its
-//     row (= dk_i), forms ds_i and its own d R_e; then the gather / scatter phase with prefetched indices.
+//     row (= dk_i), forms ds_i and its own d z_e; then the scatter phase, which reads each entry's LeakyReLU branch
+//     bits from the mask the forward stored (no y gathers: 8 B per entry at h = 64 instead of 2 x 256 B of dependent
+//     L2 reads), with the next entry's indices and mask words prefetched.
 // ------------------------------------------------------------------------------------------------
 template <int T, int LC>
 __global__ void __launch_bounds__(kFusedThreads)
@@ -779,12 +854,14 @@ __global__ void __launch_bounds__(kFusedThreads)
                           const float* __restrict__ abl_noise, const float* __restrict__ deg_w,
                           const float* __restrict__ deg_b, int hard_k, float* R, int32_t* __restrict__ rank,
                           float* __restrict__ s_out, float* __restrict__ k_out, float* __restrict__ out,
-                          float* zero_ws, long long zero_count) {
+                          uint32_t* __restrict__ branch_mask, float* __restrict__ r1_out, float* zero_ws,
+                          long long zero_count) {
   pdl_trigger();
   if constexpr (LC > 0) {
     L = LC;
     h = 16 * LC;
   }
+  const int W = (h + 31) >> 5;           // branch-mask words per entry
   extern __shared__ float sR[];          // [cap] scores of this block's entry range
   __shared__ int rng[4];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -816,11 +893,16 @@ __global__ void __launch_bounds__(kFusedThreads)
       RowSlice<T> yu, yv;
       load_slice<T>(yu, y + (size_t)u * h, h, lg, L, valid);
       load_slice<T>(yv, y + (size_t)v * h, h, lg, L, valid);
-      const float z = group_sum(edge_partial<T>(yu, yv, bias), L);
+      BranchBits<T> bb;   // formed whether or not it is stored: one code path keeps the register count of edge_partial
+      const float z = group_sum(edge_partial_bits<T>(yu, yv, bias, lg, L, bb), L);
+      if (branch_mask != nullptr) store_branch_mask<T>(bb, h, lg, L, valid, branch_mask + (size_t)(eb0 + idx) * W);
       if (valid && lg == 0) {
         const int e = eb0 + idx;
         float r = sigmoidf_(z);
-        if (abl_noise != nullptr) r = sigmoidf_(r + __ldg(abl_noise + e));  // dgm.py:1933-1935
+        if (abl_noise != nullptr) {
+          if (r1_out != nullptr) r1_out[e] = r;
+          r = sigmoidf_(r + __ldg(abl_noise + e));  // dgm.py:1933-1935
+        }
         R[e] = r;
         if (idx < cap) sR[idx] = r;
       }
@@ -872,7 +954,7 @@ template <int T, int LC>
 __global__ void __launch_bounds__(kFusedThreads, DGGB_BWD2_MIN_BLOCKS)
     dgg_bwd_fused2_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ erow,
                           const int32_t* __restrict__ col, int n, int nnz, int h, int L, int epb, int cap,
-                          const float* __restrict__ y, const float* __restrict__ be,
+                          const uint32_t* __restrict__ branch_mask, const float* __restrict__ r1_in,
                           const float* __restrict__ abl_noise, int hard_k, const float* __restrict__ R,
                           const int32_t* __restrict__ rank, const float* __restrict__ s_in,
                           const float* __restrict__ k_in, const float* __restrict__ g_out,
@@ -883,9 +965,9 @@ __global__ void __launch_bounds__(kFusedThreads, DGGB_BWD2_MIN_BLOCKS)
     L = LC;
     h = 16 * LC;
   }
-  extern __shared__ float sm2[];         // sT[cap]: d out / d k terms, sDr[cap]: d loss / d R_e   (nE <= cap, host)
+  extern __shared__ float sm2[];         // sT[cap]: d out / d k terms, sDz[cap]: d loss / d z_e   (nE <= cap, host)
   float* sT = sm2;
-  float* sDr = sm2 + cap;
+  float* sDz = sm2 + cap;
   __shared__ float dbe_s[512];           // block-level bias-gradient accumulator (h <= 512)
   __shared__ float red[2][kFusedThreads / kWarp];
   __shared__ int rng[4];
@@ -935,7 +1017,8 @@ __global__ void __launch_bounds__(kFusedThreads, DGGB_BWD2_MIN_BLOCKS)
         const float r2 = __ldg(R + e);
         dr *= r2 * (1.f - r2);  // through the second sigmoid
       }
-      sDr[idx] = dr;
+      const float r1e = __ldg(r1_in + e);   // the pre-noise sigmoid (R itself without noise)
+      sDz[idx] = dr * r1e * (1.f - r1e);
     }
     dw_acc = warp_sum(dw_acc);
     db_acc = warp_sum(db_acc);
@@ -951,10 +1034,11 @@ __global__ void __launch_bounds__(kFusedThreads, DGGB_BWD2_MIN_BLOCKS)
     for (int wv = 0; wv < kFusedThreads / kWarp; ++wv) t += red[threadIdx.x][wv];
     if (t != 0.f) atomicAdd(ddeg + threadIdx.x, t);
   }
-  // ---- phase B: per entry, recompute z and scatter d pre; every group walks a contiguous run (one flush of the
-  // source-row accumulator per row change), indices of the next entry prefetched ----
-  RowSlice<T> bias, dbe_acc, acc;
-  load_slice<T>(bias, be, h, lg, L);
+  // ---- phase B: per entry, d pre = dz LeakyReLU'(pre) from the forward's branch mask (y is not read), scattered;
+  // every group walks a contiguous run (one flush of the source-row accumulator per row change), the indices and mask
+  // words of the next entry prefetched ----
+  const int W = (h + 31) >> 5;
+  RowSlice<T> dbe_acc, acc;
 #pragma unroll
   for (int t = 0; t < T; ++t) dbe_acc.v[t] = acc.v[t] = make_float4(0.f, 0.f, 0.f, 0.f);
   const int groups = (kFusedThreads / kWarp) * G;
@@ -962,6 +1046,8 @@ __global__ void __launch_bounds__(kFusedThreads, DGGB_BWD2_MIN_BLOCKS)
   const int g0 = (warp * G + grp) * per;
   int cur_u = -1;
   int u_n = 0, v_n = 0;
+  uint32_t nib_n[T];
+  load_branch_mask<T>(nib_n, branch_mask + (size_t)(eb0 + g0) * W, h, lg, L, g0 < nE);
   if (g0 < nE) {
     u_n = __ldg(erow + eb0 + g0);
     v_n = __ldg(col + eb0 + g0);
@@ -970,17 +1056,16 @@ __global__ void __launch_bounds__(kFusedThreads, DGGB_BWD2_MIN_BLOCKS)
     const int idx = g0 + it;
     const bool valid = idx < nE;
     const int u = u_n, v = v_n;
-    if (it + 1 < per && idx + 1 < nE) {
+    uint32_t nib[T];
+#pragma unroll
+    for (int t = 0; t < T; ++t) nib[t] = nib_n[t];
+    const bool next = it + 1 < per && idx + 1 < nE;
+    if (next) {
       u_n = __ldg(erow + eb0 + idx + 1);
       v_n = __ldg(col + eb0 + idx + 1);
     }
-    const float dr = valid ? sDr[idx] : 0.f;
-    RowSlice<T> yu, yv;
-    load_slice<T>(yu, y + (size_t)u * h, h, lg, L, valid);
-    load_slice<T>(yv, y + (size_t)v * h, h, lg, L, valid);
-    const float z = group_sum(edge_partial<T>(yu, yv, bias), L);
-    const float r1s = sigmoidf_(z);
-    const float dz = valid ? dr * r1s * (1.f - r1s) : 0.f;
+    load_branch_mask<T>(nib_n, branch_mask + (size_t)(eb0 + idx + 1) * W, h, lg, L, next);
+    const float dz = valid ? sDz[idx] : 0.f;
     if (valid && u != cur_u) {  // group-uniform branch: flush the finished source row
       if (cur_u >= 0) {
 #pragma unroll
@@ -995,11 +1080,7 @@ __global__ void __launch_bounds__(kFusedThreads, DGGB_BWD2_MIN_BLOCKS)
 #pragma unroll
     for (int t = 0; t < T; ++t) {
       const int c = 4 * (lg + L * t);
-      float4 d;
-      d.x = dz * leaky_grad(yu.v[t].x - yv.v[t].x + bias.v[t].x);
-      d.y = dz * leaky_grad(yu.v[t].y - yv.v[t].y + bias.v[t].y);
-      d.z = dz * leaky_grad(yu.v[t].z - yv.v[t].z + bias.v[t].z);
-      d.w = dz * leaky_grad(yu.v[t].w - yv.v[t].w + bias.v[t].w);
+      const float4 d = branch_scale(nib[t], dz);
       dbe_acc.v[t].x += d.x; dbe_acc.v[t].y += d.y; dbe_acc.v[t].z += d.z; dbe_acc.v[t].w += d.w;
       if (valid && u != v) {  // a self loop adds +d and -d to the same row: skip both (it still counts for dbe)
         acc.v[t].x += d.x; acc.v[t].y += d.y; acc.v[t].z += d.z; acc.v[t].w += d.w;
@@ -1157,13 +1238,15 @@ extern "C" int dggb_row_firstk_bwd(const int32_t* rowptr, int32_t n, const float
   return launch_status();
 }
 
-extern "C" int dggb_dgg_edge_fwd_fused(const int32_t* rowptr, const int32_t* erow, const int32_t* col, int32_t n,
-                                       int32_t nnz, int32_t max_row_nnz, int32_t h, const float* y, const float* be,
-                                       const float* deg_w, const float* deg_b, const float* ablation_noise,
-                                       int32_t hard_k, float* R, int32_t* rank, float* s, float* k, float* out,
-                                       float* zero_ws, int64_t zero_count, void* stream) {
+extern "C" int dggb_dgg_edge_fwd_fused_mask(const int32_t* rowptr, const int32_t* erow, const int32_t* col,
+                                            int32_t n, int32_t nnz, int32_t max_row_nnz, int32_t h, const float* y,
+                                            const float* be, const float* deg_w, const float* deg_b,
+                                            const float* ablation_noise, int32_t hard_k, float* R, int32_t* rank,
+                                            float* s, float* k, float* out, uint32_t* branch_mask, float* r1,
+                                            float* zero_ws, int64_t zero_count, void* stream) {
   if (!rowptr || !erow || !col || !y || !be || !deg_w || !deg_b || !R || !rank || !s || !k || !out || n < 0 ||
-      nnz < 0 || h <= 0 || max_row_nnz < 0 || zero_count < 0)
+      nnz < 0 || h <= 0 || max_row_nnz < 0 || zero_count < 0 ||
+      (branch_mask != nullptr && ablation_noise != nullptr && r1 == nullptr))   // the backward would lack r1
     return DGGB_ERR_BAD_ARG;
   if (h % 4 != 0 || h > 512) return DGGB_ERR_BAD_SHAPE;
   if (nnz == 0 || max_row_nnz > kFusedMaxDeg) return DGGB_ERR_UNSUPPORTED;   // use the two-launch entry point
@@ -1181,8 +1264,8 @@ extern "C" int dggb_dgg_edge_fwd_fused(const int32_t* rowptr, const int32_t* ero
     const int st = allow_dynamic_smem(kern, (size_t)cap * sizeof(float));
     if (st != DGGB_OK) return st;
     launch_pdl(kern, dim3(blocks), dim3(kFusedThreads), (size_t)cap * sizeof(float), as_stream(stream), rowptr, erow,
-               col, n, nnz, h, L, epb, cap, y, be, ablation_noise, deg_w, deg_b, hard_k, R, rank, s, k, out, zero_ws,
-               (long long)zero_count);
+               col, n, nnz, h, L, epb, cap, y, be, ablation_noise, deg_w, deg_b, hard_k, R, rank, s, k, out,
+               branch_mask, r1, zero_ws, (long long)zero_count);
     return launch_status();
   };
   if (fused_v1()) {
@@ -1211,25 +1294,27 @@ extern "C" int dggb_dgg_edge_fwd_fused(const int32_t* rowptr, const int32_t* ero
   return dispatch_T(h, L, [&](auto tc) { return go(dgg_fwd_fused2_kernel<decltype(tc)::value, 0>); });
 }
 
-extern "C" int dggb_dgg_edge_bwd_fused(const int32_t* rowptr, const int32_t* erow, const int32_t* col, int32_t n,
-                                       int32_t nnz, int32_t max_row_nnz, int32_t h, const float* y, const float* be,
-                                       const float* deg_w, const float* deg_b, const float* ablation_noise,
-                                       int32_t hard_k, const float* R, const int32_t* rank, const float* s,
-                                       const float* k, const float* g_out, float* ds_ws, float* dy, float* dbe,
-                                       float* ddeg, void* stream) {
-  if (!rowptr || !erow || !col || !y || !be || !deg_w || !deg_b || !R || !rank || !s || !k || !g_out || !ds_ws ||
-      !dy || !dbe || !ddeg || n < 0 || nnz < 0 || h <= 0 || max_row_nnz < 0)
+extern "C" int dggb_dgg_edge_bwd_fused_mask(const int32_t* rowptr, const int32_t* erow, const int32_t* col,
+                                            int32_t n, int32_t nnz, int32_t max_row_nnz, int32_t h,
+                                            const float* deg_w, const float* deg_b, const float* ablation_noise,
+                                            int32_t hard_k, const float* R, const int32_t* rank, const float* s,
+                                            const float* k, const uint32_t* branch_mask, const float* r1,
+                                            const float* g_out, float* ds_ws, float* dy, float* dbe, float* ddeg,
+                                            void* stream) {
+  if (!rowptr || !erow || !col || !deg_w || !deg_b || !R || !rank || !s || !k || !branch_mask || !g_out || !ds_ws ||
+      !dy || !dbe || !ddeg || n < 0 || nnz < 0 || h <= 0 || max_row_nnz < 0 || (ablation_noise && !r1))
     return DGGB_ERR_BAD_ARG;
   if (h % 4 != 0 || h > 512) return DGGB_ERR_BAD_SHAPE;
   if (nnz == 0 || max_row_nnz > kFusedMaxDeg) return DGGB_ERR_UNSUPPORTED;
   if (n == 0) return DGGB_OK;
   const int L = lanes_per_edge(h);
+  const float* r1_in = ablation_noise ? r1 : R;   // the pre-noise sigmoid of every entry
   auto go = [&](auto kern) {
     int occ = 0, blocks, epb;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kFusedThreads, 0);
     fused_grid(nnz, occ, &blocks, &epb);
-    launch_pdl(kern, dim3(blocks), dim3(kFusedThreads), 0, as_stream(stream), rowptr, erow, col, n, nnz, h, L, epb, y,
-               be, ablation_noise, hard_k, R, rank, s, k, g_out, deg_w, deg_b, ds_ws, dy, dbe, ddeg);
+    launch_pdl(kern, dim3(blocks), dim3(kFusedThreads), 0, as_stream(stream), rowptr, erow, col, n, nnz, h, L, epb,
+               branch_mask, r1_in, ablation_noise, hard_k, R, rank, s, k, g_out, deg_w, deg_b, ds_ws, dy, dbe, ddeg);
     return launch_status();
   };
   // second generation: two shared-memory floats per entry of the block's window (epb + max_row_nnz entries); graphs
@@ -1245,8 +1330,8 @@ extern "C" int dggb_dgg_edge_bwd_fused(const int32_t* rowptr, const int32_t* ero
     const int st = allow_dynamic_smem(kern, (size_t)cap * 2 * sizeof(float));
     if (st != DGGB_OK) return st;
     launch_pdl(kern, dim3(blocks), dim3(kFusedThreads), (size_t)cap * 2 * sizeof(float), as_stream(stream), rowptr,
-               erow, col, n, nnz, h, L, epb, cap, y, be, ablation_noise, hard_k, R, rank, s, k, g_out, deg_w, deg_b,
-               ds_ws, dy, dbe, ddeg);
+               erow, col, n, nnz, h, L, epb, cap, branch_mask, r1_in, ablation_noise, hard_k, R, rank, s, k, g_out,
+               deg_w, deg_b, ds_ws, dy, dbe, ddeg);
     return launch_status();
   };
   if (!fused_v1()) {
@@ -1276,4 +1361,32 @@ extern "C" int dggb_dgg_edge_bwd_fused(const int32_t* rowptr, const int32_t* ero
     }
   }
   return dispatch_T(h, L, [&](auto tc) { return go(dgg_bwd_fused_kernel<decltype(tc)::value, 0>); });
+}
+
+// The fused entry points without the branch mask.  The forward is the masked one writing no mask.  The backward keeps
+// its arguments and its accumulate-into contract but has no mask to read: it runs the two-launch backward, which
+// recomputes the pre-activations from y (the dbe flush there uses scalar atomics, so any dbe alignment is fine).
+extern "C" int dggb_dgg_edge_fwd_fused(const int32_t* rowptr, const int32_t* erow, const int32_t* col, int32_t n,
+                                       int32_t nnz, int32_t max_row_nnz, int32_t h, const float* y, const float* be,
+                                       const float* deg_w, const float* deg_b, const float* ablation_noise,
+                                       int32_t hard_k, float* R, int32_t* rank, float* s, float* k, float* out,
+                                       float* zero_ws, int64_t zero_count, void* stream) {
+  return dggb_dgg_edge_fwd_fused_mask(rowptr, erow, col, n, nnz, max_row_nnz, h, y, be, deg_w, deg_b, ablation_noise,
+                                      hard_k, R, rank, s, k, out, nullptr, nullptr, zero_ws, zero_count, stream);
+}
+
+extern "C" int dggb_dgg_edge_bwd_fused(const int32_t* rowptr, const int32_t* erow, const int32_t* col, int32_t n,
+                                       int32_t nnz, int32_t max_row_nnz, int32_t h, const float* y, const float* be,
+                                       const float* deg_w, const float* deg_b, const float* ablation_noise,
+                                       int32_t hard_k, const float* R, const int32_t* rank, const float* s,
+                                       const float* k, const float* g_out, float* ds_ws, float* dy, float* dbe,
+                                       float* ddeg, void* stream) {
+  if (!rowptr || !erow || !col || !y || !be || !deg_w || !deg_b || !R || !rank || !s || !k || !g_out || !ds_ws ||
+      !dy || !dbe || !ddeg || n < 0 || nnz < 0 || h <= 0 || max_row_nnz < 0)
+    return DGGB_ERR_BAD_ARG;
+  if (h % 4 != 0 || h > 512) return DGGB_ERR_BAD_SHAPE;
+  if (nnz == 0 || max_row_nnz > kFusedMaxDeg) return DGGB_ERR_UNSUPPORTED;
+  if (n == 0) return DGGB_OK;
+  return dggb_dgg_edge_bwd(rowptr, erow, col, n, nnz, h, y, be, deg_w, deg_b, ablation_noise, hard_k, R, rank, s, k,
+                           g_out, ds_ws, dy, dbe, ddeg, stream);
 }

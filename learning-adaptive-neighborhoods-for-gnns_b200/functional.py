@@ -60,17 +60,22 @@ class _DGGEdge(torch.autograd.Function):
         out = torch.empty(E, dtype=torch.float32, device=dev)
         mx = graph.max_row_nnz
         fused = 0 < mx <= _FUSED_MAX_ROW and E > 0   # no hub rows: one launch per direction
-        zbuf = None
+        zbuf = mask = r1 = None
         if fused:
             if any(ctx.needs_input_grad[:4]):
                 # the backward's accumulation buffers (dy | dbe | ddeg (+pad) | ds) are cleared by the forward
                 # launch: no separate fill kernel between the two fused launches of a training step
                 zbuf = torch.empty(n * h + h + 4 + n, dtype=torch.float32, device=dev)
-            check(lib().dggb_dgg_edge_fwd_fused(p(graph.rowptr), p(graph.erow), p(graph.col), i32(n), i32(E), i32(mx),
-                                                i32(h), p(y), p(be), p(deg_w), p(deg_b), p(noise), i32(hard_k), p(R),
-                                                p(rank), p(s), p(k), p(out), p(zbuf),
-                                                i64(0 if zbuf is None else zbuf.numel()), stream()),
-                  "dgg_edge_fwd_fused")
+                # LeakyReLU branch bits of every entry (uint32 words held as int32) and, with noise, the pre-noise
+                # sigmoid: the backward reads these instead of gathering y again
+                mask = torch.empty(E, (h + 31) // 32, dtype=torch.int32, device=dev)
+                if noise is not None:
+                    r1 = torch.empty(E, dtype=torch.float32, device=dev)
+            check(lib().dggb_dgg_edge_fwd_fused_mask(p(graph.rowptr), p(graph.erow), p(graph.col), i32(n), i32(E),
+                                                     i32(mx), i32(h), p(y), p(be), p(deg_w), p(deg_b), p(noise),
+                                                     i32(hard_k), p(R), p(rank), p(s), p(k), p(out), p(mask), p(r1),
+                                                     p(zbuf), i64(0 if zbuf is None else zbuf.numel()), stream()),
+                  "dgg_edge_fwd_fused_mask")
         else:
             check(lib().dggb_dgg_edge_fwd(p(graph.rowptr), p(graph.erow), p(graph.col), i32(n), i32(E), i32(h), p(y),
                                           p(be), p(deg_w), p(deg_b), p(noise), i32(hard_k), p(R), p(rank), p(s), p(k),
@@ -78,7 +83,7 @@ class _DGGEdge(torch.autograd.Function):
         ctx.graph, ctx.hard_k, ctx.fused_mx = graph, hard_k, (mx if fused else -1)
         ctx.zbuf = zbuf
         ctx.set_materialize_grads(False)   # k / R / rank never carry gradients: no zero tensors for them per step
-        ctx.save_for_backward(y, be, deg_w, deg_b, noise, R, rank, s, k)
+        ctx.save_for_backward(y, be, deg_w, deg_b, noise, R, rank, s, k, mask, r1)
         ctx.mark_non_differentiable(k, R, rank)
         return out, k, R, rank
 
@@ -86,7 +91,7 @@ class _DGGEdge(torch.autograd.Function):
     def backward(ctx, g_out, _gk, _gR, _grank):
         if g_out is None:
             return (None,) * 7
-        y, be, deg_w, deg_b, noise, R, rank, s, k = ctx.saved_tensors
+        y, be, deg_w, deg_b, noise, R, rank, s, k, mask, r1 = ctx.saved_tensors
         g = ctx.graph
         n, h = y.shape
         # one zero-filled buffer: dy | dbe | ddeg (+pad) | ds scratch (already cleared by the fused forward launch;
@@ -100,10 +105,11 @@ class _DGGEdge(torch.autograd.Function):
         if g.nnz == 0:
             pass                             # no entries: every gradient is 0, nothing to launch
         elif ctx.fused_mx > 0:
-            check(lib().dggb_dgg_edge_bwd_fused(p(g.rowptr), p(g.erow), p(g.col), i32(n), i32(g.nnz), i32(ctx.fused_mx),
-                                                i32(h), p(y), p(be), p(deg_w), p(deg_b), p(noise), i32(ctx.hard_k),
-                                                p(R), p(rank), p(s), p(k), p(_f32c(g_out)), p(ds_ws), p(dy), p(dbe),
-                                                p(ddeg), stream()), "dgg_edge_bwd_fused")
+            check(lib().dggb_dgg_edge_bwd_fused_mask(p(g.rowptr), p(g.erow), p(g.col), i32(n), i32(g.nnz),
+                                                     i32(ctx.fused_mx), i32(h), p(deg_w), p(deg_b), p(noise),
+                                                     i32(ctx.hard_k), p(R), p(rank), p(s), p(k), p(mask), p(r1),
+                                                     p(_f32c(g_out)), p(ds_ws), p(dy), p(dbe), p(ddeg), stream()),
+                  "dgg_edge_bwd_fused_mask")
         else:
             check(lib().dggb_dgg_edge_bwd(p(g.rowptr), p(g.erow), p(g.col), i32(n), i32(g.nnz), i32(h), p(y), p(be),
                                           p(deg_w), p(deg_b), p(noise), i32(ctx.hard_k), p(R), p(rank), p(s), p(k),
