@@ -113,8 +113,7 @@ int dggb_dgg_edge_bwd(const int32_t* rowptr, const int32_t* erow, const int32_t*
  * shared memory and runs both phases back to back.  Same arguments.  R and rank are the two-launch results bit for
  * bit; s, k, out and the gradients differ from them by the summation order of the row sums (and of the atomics).
  * Return DGGB_ERR_UNSUPPORTED when max_row_nnz > 512 or nnz == 0: call the two-launch entry point instead.
- * DGGB_FUSED_EPB (read per call; values below 1 are ignored) sets the smallest number of entries per block, and
- * DGGB_FUSED_V1 selects the first-generation kernels (see csrc/dgg_edge.cu).
+ * DGGB_FUSED_EPB (read per call; values below 1 are ignored) sets the smallest number of entries per block.
  *
  * Training goes through the _mask pair.  The forward also stores what the backward would otherwise recompute from y:
  *   branch_mask [E, ceil(H/32)] uint32: bit c % 32 of word c / 32 is set when pre_c = y_u - y_v + be > 0;

@@ -3,7 +3,8 @@
 // row sum -> Linear(1,1) -> N-long row sort -> tanh first-k -> un-sort scatter -> to_sparse).
 //
 // Graphs without hub rows (longest row <= 512 entries: Cora, Citeseer, Pubmed): ONE launch per direction, a block
-// owning a contiguous range of rows and their edges (dgg_fwd_fused_kernel / dgg_bwd_fused_kernel below).
+// owning a contiguous range of rows and their edges (dgg_fwd_fused2_kernel; backward dgg_bwd_fused2_kernel, or
+// dgg_bwd_fused_kernel for block windows above 6 144 entries).
 // Graphs with hub rows: two launches per direction so that a power-law hub cannot serialise a warp:
 //   fwd:  edge_score (edge-parallel, perfectly balanced)  ->  row_rank (warp per CSR row)
 //   bwd:  row_dk     (warp per CSR row)                    ->  edge_grad (edge-parallel, vector reds)
@@ -203,11 +204,11 @@ __device__ __forceinline__ bool stage_row(const float* __restrict__ R, float* sr
 constexpr int kLongThreads = 256;
 constexpr int kLongTile = 2048;
 
-__device__ __forceinline__ float first_k_tanh_(float r, float k) { return 1.f - 0.5f * (1.f + tanhf(r - k)); }
+__device__ __forceinline__ float first_k_tanh(float r, float k) { return 1.f - 0.5f * (1.f + tanhf(r - k)); }
 
 __device__ __forceinline__ float ranked_value(int mode, float v, int r, float k, int hard_k) {
   if (mode == 3) return r < hard_k ? v : 0.f;
-  const float fk = first_k_tanh_((float)r, k);
+  const float fk = first_k_tanh((float)r, k);
   return mode == 0 ? v * fk : (mode == 1 ? fk : v * (fk + 1.f));
 }
 
@@ -464,8 +465,6 @@ __global__ void __launch_bounds__(kEdgeWarps* kWarp)
 //   fk(r) = 1 - 0.5 * (1 + tanh(r - k_i));  mode 0: out = score * fk (k_times_edge_prob)
 // Off-support entries are exact zeros that sort after every positive score, so in-row ranks are exact.
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ float first_k_tanh(float r, float k) { return 1.f - 0.5f * (1.f + tanhf(r - k)); }
-
 __global__ void __launch_bounds__(kEdgeWarps* kWarp)
     row_firstk_fwd_kernel(const int32_t* __restrict__ rowptr, int n, const float* __restrict__ score,
                           const float* __restrict__ k_in, int mode, int32_t* __restrict__ rank,
@@ -518,11 +517,12 @@ __global__ void __launch_bounds__(kEdgeWarps* kWarp)
 }
 
 // ------------------------------------------------------------------------------------------------
-// Fused variants for graphs without hub rows (max row length <= kFusedMaxDeg): ONE launch per direction.
+// Fused kernels for graphs without hub rows (max row length <= kFusedMaxDeg): ONE launch per direction.
 // Block b owns the CSR rows that START inside the edge interval [b*epb, (b+1)*epb) -- found from erow in two
 // dependent loads, no search -- and therefore the contiguous edge range [rowptr[r0], rowptr[r1]) of at most
-// epb + max_deg entries.  fwd: edge-parallel scores into shared memory -> __syncthreads -> warp-per-row rank from
-// shared memory.  bwd: warp-per-row dk/ds into shared memory -> __syncthreads -> edge-parallel gradients.
+// epb + max_deg entries (the block's window).  The forward is always dgg_fwd_fused2_kernel.  The backward is
+// dgg_bwd_fused2_kernel when the window holds at most 6 144 entries (two shared-memory floats per entry), and
+// dgg_bwd_fused_kernel, which keeps only per-row values in shared memory, for larger windows.
 // At Pubmed shape the two-launch path is pure latency (2 x ~12 us for 0.4 MB of edge data); this is one wave of
 // blocks with ~4 dependent memory round trips.  R and rank are bit-identical to the two-launch kernels; s, k and
 // out differ from them by the summation order of the row sums.
@@ -552,131 +552,9 @@ __device__ __forceinline__ void fused_row_range(const int32_t* __restrict__ rowp
 // LC > 0: lanes per edge and the hidden width (h == 16 * LC, T == 4) are compile-time constants, which folds every
 // `chunk < h` guard, the zero fills of out-of-range chunks and the per-chunk address arithmetic (static SASS of the
 // runtime-L version: ~270 instructions per edge slot, a third of them guards / CS2R / IMAD).
-template <int T, int LC>
-__global__ void __launch_bounds__(kFusedThreads)
-    dgg_fwd_fused_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ erow,
-                         const int32_t* __restrict__ col, int n, int nnz, int h, int L, int epb, int cap,
-                         const float* __restrict__ y, const float* __restrict__ be,
-                         const float* __restrict__ abl_noise, const float* __restrict__ deg_w,
-                         const float* __restrict__ deg_b, int hard_k, float* R, int32_t* __restrict__ rank,
-                         float* __restrict__ s_out, float* __restrict__ k_out, float* __restrict__ out,
-                         uint32_t* __restrict__ branch_mask, float* __restrict__ r1_out, float* zero_ws,
-                         long long zero_count) {
-  pdl_trigger();
-  if constexpr (LC > 0) {
-    L = LC;
-    h = 16 * LC;
-  }
-  const int W = (h + 31) >> 5;           // branch-mask words per entry
-  extern __shared__ float sR[];          // [cap] scores of this block's edge range
-  __shared__ int rng[4];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int G = kWarp / L, lg = lane % L, grp = lane / L;
-  pdl_wait();
-  zero_fill(zero_ws, zero_count);   // the backward's accumulation buffers (dy | dbe | ddeg | ds)
-  fused_row_range(rowptr, erow, n, nnz, epb, rng);
-  const int r0 = rng[0], r1 = rng[1], eb0 = rng[2], eb1 = rng[3];
-  const int nE = eb1 - eb0;
-  // ---- phase 1: every group of L lanes walks a contiguous run of edges ----
-  {
-    RowSlice<T> bias;
-    load_slice<T>(bias, be, h, lg, L);
-    const int groups = (kFusedThreads / kWarp) * G;
-    const int per = (nE + groups - 1) / groups;
-    const int g0 = (warp * G + grp) * per;
-#pragma unroll 1   // unrolled, the branch-mask bits push ptxas into small spills
-    for (int it = 0; it < per; ++it) {
-      const int idx = g0 + it;
-      const bool valid = idx < nE;
-      const int e = eb0 + (valid ? idx : 0);
-      const int u = valid ? __ldg(erow + e) : 0, v = valid ? __ldg(col + e) : 0;
-      RowSlice<T> yu, yv;
-      load_slice<T>(yu, y + (size_t)u * h, h, lg, L, valid);
-      load_slice<T>(yv, y + (size_t)v * h, h, lg, L, valid);
-      BranchBits<T> bb;   // formed whether or not it is stored: one code path keeps the register count of edge_partial
-      const float z = group_sum(edge_partial_bits<T>(yu, yv, bias, lg, L, bb), L);
-      if (branch_mask != nullptr) store_branch_mask<T>(bb, h, lg, L, valid, branch_mask + (size_t)e * W);
-      if (valid && lg == 0) {
-        float r = sigmoidf_(z);
-        if (abl_noise != nullptr) {
-          if (r1_out != nullptr) r1_out[e] = r;
-          r = sigmoidf_(r + __ldg(abl_noise + e));  // dgm.py:1933-1935
-        }
-        R[e] = r;
-        if (idx < cap) sR[idx] = r;
-      }
-    }
-  }
-  __syncthreads();
-  // ---- phase 2: 8 lanes per row (the average row has ~6 entries), four rows per warp at a time.  The rank is a
-  // count over the row (deg^2 compares): rows longer than kLongRow would leave one 8-lane group running long after
-  // the rest of the grid has finished (152-entry row: ~25 us), so they only get s and k here and are ranked by the
-  // whole block afterwards. ----
-  constexpr int kLongRow = 32, kLongCap = 32;
-  __shared__ int long_rows[kLongCap];
-  __shared__ float long_k[kLongCap];
-  __shared__ int n_long;
-  if (threadIdx.x == 0) n_long = 0;
-  __syncthreads();
-  const float w = __ldg(deg_w), b = __ldg(deg_b);
-  const int sub = lane >> 3, sl = lane & 7;
-  auto rank_entries = [&](int beg, int deg, float k, bool in_s, int first, int stride) {
-    const float* srow = sR + (beg - eb0);
-    for (int m = first; m < deg; m += stride) {
-      const float mine = in_s ? srow[m] : __ldcg(R + beg + m);
-      int cnt = 0;
-      if (in_s) {
-#pragma unroll 4
-        for (int j = 0; j < deg; ++j) {
-          const float rj = srow[j];
-          cnt += (rj > mine) || (rj == mine && j < m);
-        }
-      } else {
-#pragma unroll 4
-        for (int j = 0; j < deg; ++j) {
-          const float rj = __ldcg(R + beg + j);
-          cnt += (rj > mine) || (rj == mine && j < m);
-        }
-      }
-      rank[beg + m] = cnt;
-      out[beg + m] = (hard_k >= 0) ? (cnt < hard_k ? mine : 0.f) : mine * first_k_plus_one((float)cnt, k);
-    }
-  };
-  for (int i0 = r0 + warp * 4; i0 < r1; i0 += (kFusedThreads / kWarp) * 4) {
-    const int i = i0 + sub;
-    const bool rv = i < r1;
-    const int beg = rv ? __ldg(rowptr + i) : eb0, end = rv ? __ldg(rowptr + i + 1) : eb0, deg = end - beg;
-    const bool in_s = (end - eb0) <= cap;
-    const float* srow = sR + (beg - eb0);
-    float s = 0.f;
-    for (int e = sl; e < deg; e += 8) s += in_s ? srow[e] : __ldcg(R + beg + e);
-    s += __shfl_xor_sync(0xffffffffu, s, 4);
-    s += __shfl_xor_sync(0xffffffffu, s, 2);
-    s += __shfl_xor_sync(0xffffffffu, s, 1);
-    const float k = leaky(w * s + b);  // dgm.py:1791-1792
-    int slot = -1;
-    if (deg > kLongRow && sl == 0) slot = atomicAdd(&n_long, 1);
-    slot = __shfl_sync(0xffffffffu, slot, lane & ~7);          // outside any divergent branch
-    const bool deferred = deg > kLongRow && slot < kLongCap;    // list full: rank it here (slow but correct)
-    if (deferred && sl == 0) {
-      long_rows[slot] = i;
-      long_k[slot] = k;
-    }
-    if (!deferred) rank_entries(beg, deg, k, in_s, sl, 8);
-    if (rv && sl == 0) {
-      s_out[i] = s;
-      k_out[i] = k;
-    }
-  }
-  __syncthreads();
-  const int nl = min(n_long, kLongCap);
-  for (int q = 0; q < nl; ++q) {
-    const int i = long_rows[q];
-    const int beg = __ldg(rowptr + i), end = __ldg(rowptr + i + 1);
-    rank_entries(beg, end - beg, long_k[q], (end - eb0) <= cap, threadIdx.x, kFusedThreads);
-  }
-}
-
+//
+// Backward for windows above 6 144 entries: warp-per-row dk / ds (the first kFusedRowsCap rows' ds in shared memory,
+// the rest through ds_ws) -> __syncthreads -> edge-parallel gradients.
 template <int T, int LC>
 __global__ void __launch_bounds__(kFusedThreads)
     dgg_bwd_fused_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ erow,
@@ -826,15 +704,15 @@ __global__ void __launch_bounds__(kFusedThreads)
   for (int c = threadIdx.x; c < h; c += kFusedThreads) atomicAdd(dbe + c, dbe_s[c]);
 }
 
-#ifndef DGGB_BWD2_MIN_BLOCKS
-#define DGGB_BWD2_MIN_BLOCKS 1
-#endif
 // ------------------------------------------------------------------------------------------------
-// Second generation of the fused kernels (same contract, same results up to the summation order of the row sums).
-// What the ncu source view of the first generation showed at Pubmed shape (profiles/r02_fused_edge_v2.md): a third
-// of the stall samples sat at block barriers (rows dealt to 8-lane groups finish at very different times, and rows
-// longer than 32 entries were ranked by the whole block after yet another barrier), a quarter behind the per-edge
-// dependent chain "index load -> gather" that every group repeated `per` times back to back.  Here
+// Second generation of the fused kernels: the forward for every window, the backward for windows of at most 6 144
+// entries (the backward has the contract of dgg_bwd_fused_kernel and its results up to the summation order of the
+// row sums).
+// Why they are entry-parallel: the ncu source view of the row-parallel design that dgg_bwd_fused_kernel keeps, at
+// Pubmed shape (profiles/r02_fused_edge_v2.md), put a third of the stall samples at block barriers (rows dealt to
+// 8-lane groups finish at very different times, and rows longer than 32 entries were ranked by the whole block after
+// yet another barrier), a quarter behind the per-edge dependent chain "index load -> gather" that every group
+// repeated `per` times back to back.  Here
 //   * phase 1 walks the block's entries INTERLEAVED over the groups (coalesced index loads) and loads the indices of
 //     the next entry while the current entry's rows are in flight: one memory round trip per entry instead of two;
 //   * phase 2 is ENTRY-parallel: thread == entry; it sweeps its own row in shared memory, which yields the rank (a
@@ -950,8 +828,10 @@ __global__ void __launch_bounds__(kFusedThreads)
   }
 }
 
+// Keep the minimum of 1 block per SM: with __launch_bounds__(kFusedThreads) alone, ptxas limits <4,4> to 64 registers
+// instead of 78 and compiles every instantiation differently.
 template <int T, int LC>
-__global__ void __launch_bounds__(kFusedThreads, DGGB_BWD2_MIN_BLOCKS)
+__global__ void __launch_bounds__(kFusedThreads, 1)
     dgg_bwd_fused2_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ erow,
                           const int32_t* __restrict__ col, int n, int nnz, int h, int L, int epb, int cap,
                           const uint32_t* __restrict__ branch_mask, const float* __restrict__ r1_in,
@@ -1136,6 +1016,24 @@ static void fused_grid(int nnz, int blocks_per_sm, int* blocks, int* epb) {
   *blocks = (nnz + *epb - 1) / *epb;
 }
 
+// instantiation of the fused kernels for hidden width h: fn(T, LC) with both as std::integral_constant, <4, L> for the
+// usual widths h == 16 L (fully specialised), dispatch_T's runtime-L <T, 0> otherwise
+template <typename F>
+static int dispatch_fused(int h, int L, F&& fn) {
+  using I4 = std::integral_constant<int, 4>;
+  if (h == 16 * L) {
+    switch (L) {
+      case 1: return fn(I4{}, std::integral_constant<int, 1>{});
+      case 2: return fn(I4{}, std::integral_constant<int, 2>{});
+      case 4: return fn(I4{}, std::integral_constant<int, 4>{});
+      case 8: return fn(I4{}, std::integral_constant<int, 8>{});
+      case 16: return fn(I4{}, std::integral_constant<int, 16>{});
+      default: return fn(I4{}, std::integral_constant<int, 32>{});
+    }
+  }
+  return dispatch_T(h, L, [&](auto tc) { return fn(tc, std::integral_constant<int, 0>{}); });
+}
+
 // Without an opt-in a block gets at most 48 KB of shared memory, static and dynamic together: the largest score
 // windows (12 288 floats in the forward, 2 x 6 144 in the backward) plus the kernels' static arrays exceed it.  The
 // opt-in is only requested for large windows, so the small graphs' launches make no extra call.
@@ -1144,9 +1042,6 @@ static int allow_dynamic_smem(K kern, size_t smem) {
   if (smem <= 40 * 1024) return DGGB_OK;
   return cuda_status(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 }
-
-// DGGB_FUSED_V1=1: first-generation fused kernels (A/B measurements); read per call, like DGGB_FUSED_EPB
-static bool fused_v1() { return getenv("DGGB_FUSED_V1") != nullptr; }
 
 static int edges_grid(long long nnz, int blocks_per_sm = 8) {
   long long need = (nnz + kEdgeWarps * kWarp - 1) / (kEdgeWarps * kWarp);
@@ -1252,14 +1147,15 @@ extern "C" int dggb_dgg_edge_fwd_fused_mask(const int32_t* rowptr, const int32_t
   if (nnz == 0 || max_row_nnz > kFusedMaxDeg) return DGGB_ERR_UNSUPPORTED;   // use the two-launch entry point
   if (n == 0) return DGGB_OK;
   const int L = lanes_per_edge(h);
-  auto go = [&](auto kern) {
+  return dispatch_fused(h, L, [&](auto tc, auto lc) {
+    auto kern = dgg_fwd_fused2_kernel<decltype(tc)::value, decltype(lc)::value>;
     int occ = 0, blocks, epb;
     // the shared-memory slice depends on epb, which depends on the occupancy: size it for the smallest grid first
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kFusedThreads,
                                                   (size_t)(128 + max_row_nnz) * sizeof(float));
     fused_grid(nnz, occ, &blocks, &epb);
     // shared-memory score window: entries beyond it (bounded-degree graphs with > ~7 M entries make epb large)
-    // are re-read from global memory by the rank phase (the `idx < cap` / `in_s` guards of the kernel)
+    // are re-read from global memory by the rank phase (the `je <= cap` / `idx < cap` guards of the kernel)
     const int cap = min(epb + max_row_nnz, 12288);
     const int st = allow_dynamic_smem(kern, (size_t)cap * sizeof(float));
     if (st != DGGB_OK) return st;
@@ -1267,31 +1163,7 @@ extern "C" int dggb_dgg_edge_fwd_fused_mask(const int32_t* rowptr, const int32_t
                col, n, nnz, h, L, epb, cap, y, be, ablation_noise, deg_w, deg_b, hard_k, R, rank, s, k, out,
                branch_mask, r1, zero_ws, (long long)zero_count);
     return launch_status();
-  };
-  if (fused_v1()) {
-    if (h == 16 * L) {   // the usual hidden widths: fully specialised kernels
-      switch (L) {
-        case 1: return go(dgg_fwd_fused_kernel<4, 1>);
-        case 2: return go(dgg_fwd_fused_kernel<4, 2>);
-        case 4: return go(dgg_fwd_fused_kernel<4, 4>);
-        case 8: return go(dgg_fwd_fused_kernel<4, 8>);
-        case 16: return go(dgg_fwd_fused_kernel<4, 16>);
-        default: return go(dgg_fwd_fused_kernel<4, 32>);
-      }
-    }
-    return dispatch_T(h, L, [&](auto tc) { return go(dgg_fwd_fused_kernel<decltype(tc)::value, 0>); });
-  }
-  if (h == 16 * L) {
-    switch (L) {
-      case 1: return go(dgg_fwd_fused2_kernel<4, 1>);
-      case 2: return go(dgg_fwd_fused2_kernel<4, 2>);
-      case 4: return go(dgg_fwd_fused2_kernel<4, 4>);
-      case 8: return go(dgg_fwd_fused2_kernel<4, 8>);
-      case 16: return go(dgg_fwd_fused2_kernel<4, 16>);
-      default: return go(dgg_fwd_fused2_kernel<4, 32>);
-    }
-  }
-  return dispatch_T(h, L, [&](auto tc) { return go(dgg_fwd_fused2_kernel<decltype(tc)::value, 0>); });
+  });
 }
 
 extern "C" int dggb_dgg_edge_bwd_fused_mask(const int32_t* rowptr, const int32_t* erow, const int32_t* col,
@@ -1309,58 +1181,33 @@ extern "C" int dggb_dgg_edge_bwd_fused_mask(const int32_t* rowptr, const int32_t
   if (n == 0) return DGGB_OK;
   const int L = lanes_per_edge(h);
   const float* r1_in = ablation_noise ? r1 : R;   // the pre-noise sigmoid of every entry
-  auto go = [&](auto kern) {
-    int occ = 0, blocks, epb;
+  return dispatch_fused(h, L, [&](auto tc, auto lc) {
+    constexpr int T = decltype(tc)::value, LC = decltype(lc)::value;
+    // second generation: two shared-memory floats per entry of the block's window (epb + max_row_nnz entries), as
+    // long as the window its one-wave grid gives fits 48 KB
+    auto kern2 = dgg_bwd_fused2_kernel<T, LC>;
+    int occ2 = 0, blocks, epb;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ2, kern2, kFusedThreads,
+                                                  (size_t)(128 + max_row_nnz) * 2 * sizeof(float));
+    fused_grid(nnz, occ2, &blocks, &epb);
+    const int cap = epb + max_row_nnz;
+    if (cap <= 6144) {
+      const int st = allow_dynamic_smem(kern2, (size_t)cap * 2 * sizeof(float));
+      if (st != DGGB_OK) return st;
+      launch_pdl(kern2, dim3(blocks), dim3(kFusedThreads), (size_t)cap * 2 * sizeof(float), as_stream(stream),
+                 rowptr, erow, col, n, nnz, h, L, epb, cap, branch_mask, r1_in, ablation_noise, hard_k, R, rank, s, k,
+                 g_out, deg_w, deg_b, ds_ws, dy, dbe, ddeg);
+      return launch_status();
+    }
+    // larger windows: dgg_bwd_fused_kernel, on the grid of its own occupancy
+    auto kern = dgg_bwd_fused_kernel<T, LC>;
+    int occ = 0;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kFusedThreads, 0);
     fused_grid(nnz, occ, &blocks, &epb);
     launch_pdl(kern, dim3(blocks), dim3(kFusedThreads), 0, as_stream(stream), rowptr, erow, col, n, nnz, h, L, epb,
                branch_mask, r1_in, ablation_noise, hard_k, R, rank, s, k, g_out, deg_w, deg_b, ds_ws, dy, dbe, ddeg);
     return launch_status();
-  };
-  // second generation: two shared-memory floats per entry of the block's window (epb + max_row_nnz entries); graphs
-  // whose one-wave grid makes that window larger than 48 KB stay on the first generation
-  auto go2 = [&](auto kern, int* fits) {
-    int occ = 0, blocks, epb;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kFusedThreads,
-                                                  (size_t)(128 + max_row_nnz) * 2 * sizeof(float));
-    fused_grid(nnz, occ, &blocks, &epb);
-    const int cap = epb + max_row_nnz;
-    *fits = cap <= 6144;
-    if (!*fits) return (int)DGGB_OK;
-    const int st = allow_dynamic_smem(kern, (size_t)cap * 2 * sizeof(float));
-    if (st != DGGB_OK) return st;
-    launch_pdl(kern, dim3(blocks), dim3(kFusedThreads), (size_t)cap * 2 * sizeof(float), as_stream(stream), rowptr,
-               erow, col, n, nnz, h, L, epb, cap, branch_mask, r1_in, ablation_noise, hard_k, R, rank, s, k, g_out,
-               deg_w, deg_b, ds_ws, dy, dbe, ddeg);
-    return launch_status();
-  };
-  if (!fused_v1()) {
-    int fits = 0, rc;
-    if (h == 16 * L) {
-      switch (L) {
-        case 1: rc = go2(dgg_bwd_fused2_kernel<4, 1>, &fits); break;
-        case 2: rc = go2(dgg_bwd_fused2_kernel<4, 2>, &fits); break;
-        case 4: rc = go2(dgg_bwd_fused2_kernel<4, 4>, &fits); break;
-        case 8: rc = go2(dgg_bwd_fused2_kernel<4, 8>, &fits); break;
-        case 16: rc = go2(dgg_bwd_fused2_kernel<4, 16>, &fits); break;
-        default: rc = go2(dgg_bwd_fused2_kernel<4, 32>, &fits); break;
-      }
-    } else {
-      rc = dispatch_T(h, L, [&](auto tc) { return go2(dgg_bwd_fused2_kernel<decltype(tc)::value, 0>, &fits); });
-    }
-    if (fits || rc != DGGB_OK) return rc;
-  }
-  if (h == 16 * L) {
-    switch (L) {
-      case 1: return go(dgg_bwd_fused_kernel<4, 1>);
-      case 2: return go(dgg_bwd_fused_kernel<4, 2>);
-      case 4: return go(dgg_bwd_fused_kernel<4, 4>);
-      case 8: return go(dgg_bwd_fused_kernel<4, 8>);
-      case 16: return go(dgg_bwd_fused_kernel<4, 16>);
-      default: return go(dgg_bwd_fused_kernel<4, 32>);
-    }
-  }
-  return dispatch_T(h, L, [&](auto tc) { return go(dgg_bwd_fused_kernel<decltype(tc)::value, 0>); });
+  });
 }
 
 // The fused entry points without the branch mask.  The forward is the masked one writing no mask.  The backward keeps

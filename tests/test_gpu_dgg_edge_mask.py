@@ -4,12 +4,11 @@ The forward stores, per entry, one bit per channel (pre_c = y_u - y_v + be > 0, 
 ablation noise, the pre-noise sigmoid r1; the backward reads them instead of gathering y.  Checked here:
 
 * the mask against a torch recomputation of pre (exact: the inputs of test_gpu_dgg_edge_paths keep every pre_c at
-  least q / 2 away from 0), for h = 4, 12, 64, 100 and 512, with and without noise, with hard_k, from both forward
-  generations; r1 against the R of the same forward without noise, bit for bit; and R, rank, s, k, out against the
-  forward without a mask, bit for bit;
+  least q / 2 away from 0), for h = 4, 12, 64, 100 and 512, with and without noise, with hard_k; r1 against the R of
+  the same forward without noise, bit for bit; and R, rank, s, k, out against the forward without a mask, bit for bit;
 * the masked backward against the unmasked entry point (which runs the two-launch backward from y): both within the
-  fp64 bounds of test_gpu_dgg_edge_paths, on the second-generation backward and on the first-generation one that
-  takes windows above 6 144 entries;
+  fp64 bounds of test_gpu_dgg_edge_paths, on dgg_bwd_fused2_kernel and on dgg_bwd_fused_kernel, which takes windows
+  above 6 144 entries;
 * argument checks of the two entry points (CPU).
 """
 import ctypes
@@ -18,7 +17,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.test_gpu_dgg_edge_paths import W, _d, _prepare, _set_path, check_grads, grad_bounds
+from tests.test_gpu_dgg_edge_paths import W, _bwd2_fits, _d, _prepare, _set_path, check_grads, grad_bounds
 
 gpu = pytest.mark.gpu
 
@@ -60,11 +59,11 @@ def _fwd(g, y, be, b, noise, hard_k, masked):
 
 MASK_CASES = [
     # (h, hard_k, noise, mode): every lane layout of the fused kernels (L = 1 .. 32, T = 1, 2, 4, h not 16 L)
-    (4, -1, False, "auto"), (4, -1, True, "v1"),
+    (4, -1, False, "auto"), (4, -1, True, "auto"),
     (12, 3, False, "auto"), (12, -1, True, "auto"),
-    (64, -1, False, "auto"), (64, -1, True, "auto"), (64, 1, False, "v1"), (64, -1, True, "v1"),
+    (64, -1, False, "auto"), (64, -1, True, "auto"), (64, 1, False, "auto"),
     (100, -1, False, "auto"), (100, 3, True, "auto"),
-    (512, -1, False, "auto"), (512, 0, True, "auto"), (512, -1, False, "v1"),
+    (512, -1, False, "auto"), (512, 0, True, "auto"),
 ]
 
 
@@ -118,9 +117,9 @@ BWD_CASES = [
     ("mixed", 64, -1, True, "auto", None, "fused2"),
     ("mixed", 100, 3, False, "auto", None, "fused2"),
     ("blocks", 16, -1, True, "auto", 64, "fused2"),
-    ("mixed", 8, 1, True, "v1", None, "fused"),
-    ("mixed", 512, -1, False, "v1", None, "fused"),
-    ("wide", 20, -1, False, "auto", 16000, "fused"),      # window above 6 144 entries: the first generation
+    ("mixed", 8, 1, True, "auto", 16000, "fused"),        # windows above 6 144 entries: dgg_bwd_fused_kernel
+    ("mixed", 512, -1, False, "auto", 16000, "fused"),
+    ("wide", 20, -1, False, "auto", 16000, "fused"),
     ("wide", 64, 2, True, "auto", 16000, "fused"),
 ]
 
@@ -133,6 +132,7 @@ def test_masked_backward_matches_the_unmasked_entry_point(graph, h, hard_k, nois
     c = _d(graph, h, hard_k, noise=noise, mode=mode, epb=epb, seed=95 + h)
     g, y, be, nz, gout, f, b = _prepare(c)
     _set_path(monkeypatch, c)
+    assert _bwd2_fits(g.nnz, g.max_row, epb) == (kernel == "fused2")
     R, rank, s, k, out, mask, r1 = _fwd(g, y, be, b, nz, hard_k, masked=True)
     ref, bounds = grad_bounds(g, f, hard_k, nz, rank, gout, y.double(), be.double())
     new = _bwd(g, y, be, b, nz, hard_k, R, rank, s, k, gout, mask, r1)

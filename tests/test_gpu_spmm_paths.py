@@ -656,7 +656,10 @@ def test_dispatch_launches_the_tabled_kernels(monkeypatch, tmp_path):
             runs.append((c, g, _stack_inputs(c, g)))
     want = []
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        torch.ones(1, device="cuda").add_(1)       # the trace can miss the first kernel after the profiler starts
+        # A profiler session that is not the process's first can lose its first few kernel records (2 or 3 of
+        # them late in a full GPU test session): untracked kernels absorb the loss before the tabled launches.
+        for _ in range(32):
+            torch.ones(1, device="cuda").add_(1)
         torch.cuda.synchronize()
         for run, (_, launches) in zip(runs, PATHS):
             c, g = run[:2]
