@@ -408,7 +408,9 @@ int dggb_gemm_tn_tc_presplit(const float* a_t_hi, const float* a_t_lo, int32_t n
  *   workspace: dggb_allpairs_workspace_bytes(n, d) bytes (hi/lo split of z + squared norms).
  *   out_rowsum (optional): sum_j exp(y_ij * inv_temp) over ALL n columns -- the normaliser of the
  *          evaluation branch softmax(log_p / temp) (dgm.py:298), accumulated in the same pass.
- * Requires d <= 128, kc <= 64.
+ * Requires kc <= 64; any d.  For d > 128 (d rounded up to 32) a k-block-streamed kernel runs the call: the query
+ *   tile is streamed 32 features at a time with each key tile, so shared memory does not depend on d.  It runs
+ *   unsplit; DGGB_AP_V1 and DGGB_AP_PARTS have no effect on it.
  *   Column parts: when the row blocks of a call fill the SMs badly (a row-sharded rank: 228 blocks on 148 SMs), the
  *   column range is cut into up to 8 parts scored by separate CTAs and a merge launch picks the best kc of a row's
  *   parts (same order, identical result).  That needs parts * row_count * kc * 8 more workspace bytes:

@@ -127,22 +127,27 @@ struct APSmem {  // byte offsets from the 1024-aligned base
   uint32_t a_hi, a_lo, b0, b_stage_bytes, nrm, vals, idx, qv, qi, bars, total;
 };
 
+// kb == 0: the k-block-streamed shape (d > 128).  No resident query tile: a stage is ONE 32-feature k-block of both
+// operands, [A_hi 128 rows | A_lo 128 rows | B_hi 64 rows | B_lo 64 rows] x 128 B, and the column norms get a ring of
+// kNrmSlots slots of their own (a stage is recycled long before the epilogue reads its tile).
+constexpr int kNrmSlots = 4;
+
 __host__ __device__ inline APSmem ap_smem_layout(int kb, int split, int stages, int kc) {
   APSmem L;
   const uint32_t a_bytes = kb * kBM * 128;  // [128 rows][128 B] per k-block
-  const uint32_t b_bytes = kb * kBN * 128;
+  const uint32_t b_bytes = kb == 0 ? (kBM + kBN) * 128 : kb * kBN * 128;
   uint32_t off = 0;
   L.a_hi = off; off += a_bytes;
   L.a_lo = off; off += (split == 3 ? a_bytes : 0);
   L.b0 = off;
   L.b_stage_bytes = b_bytes * (split == 3 ? 2 : 1);
   off += L.b_stage_bytes * stages;
-  L.nrm = off; off += stages * kBN * 4;
+  L.nrm = off; off += (kb == 0 ? kNrmSlots : stages) * kBN * 4;
   L.vals = off; off += kc * kBM * 4;
   L.idx = off; off += kc * kBM * 4;
   L.qv = off; off += kQCap * kBM * 4;
   L.qi = off; off += kQCap * kBM * 4;
-  L.bars = off; off += 128;
+  L.bars = off; off += kb == 0 ? 256 : 128;
   L.total = off;
   return L;
 }
@@ -249,6 +254,10 @@ __device__ __forceinline__ float merge_row(float* Lv, int32_t* Li, const float* 
 }
 
 // NOISE: 0 none, 1 injected tensor, 2 Philox Gumbel(0, noise_scale), 3 none + softmax normaliser (out_rowsum)
+// KB = 0: the k-block-streamed instantiation for d > 128 (kblocks = dpad / 32 k-blocks, given at run time).  The query
+// tile is loaded again with every key tile, one k-block per stage, so shared memory does not depend on d.  A stage is
+// released by the MMA commit alone; the column norms travel in their own ring (nfull / nempty, kNrmSlots slots) that
+// the epilogue releases.  Everything else, the epilogue included, is the code of the resident-tile instantiations.
 template <int KB, int SPLIT, int NOISE>
 __global__ void __launch_bounds__(kAPThreads, 1)
     allpairs_topk_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
@@ -257,7 +266,7 @@ __global__ void __launch_bounds__(kAPThreads, 1)
                          unsigned long long seed, float noise_scale, int kc, int stages,
                          int32_t* __restrict__ out_idx, float* __restrict__ out_val, float inv_temp,
                          float* __restrict__ out_rowsum, const float* __restrict__ after_val,
-                         const int32_t* __restrict__ after_idx) {
+                         const int32_t* __restrict__ after_idx, int kblocks) {
   extern __shared__ uint8_t smem_raw[];
   // 1024-B align WITHOUT laundering the pointer through an integer (keeps it a shared-space pointer, so
   // every access below compiles to LDS/STS instead of generic LD/ST)
@@ -265,11 +274,13 @@ __global__ void __launch_bounds__(kAPThreads, 1)
   const APSmem L = ap_smem_layout(KB, SPLIT, stages, kc);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L.bars);
   uint64_t* full = bars;            // [stages]  TMA -> MMA/epilogue
-  uint64_t* empty = bars + 4;       // [stages]  MMA + 4 epilogue warps -> TMA
+  uint64_t* empty = bars + 4;       // [stages]  MMA + 4 epilogue warps -> TMA  (KB = 0: MMA alone)
   uint64_t* tfull = bars + 8;       // [2]       MMA -> epilogue
   uint64_t* tempty = bars + 10;     // [2]       epilogue -> MMA
   uint64_t* afull = bars + 12;      // A tile landed
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 13);
+  uint64_t* nfull = bars + 14;      // KB = 0: [kNrmSlots]  column norms of a tile landed
+  uint64_t* nempty = bars + 18;     // KB = 0: [kNrmSlots]  4 epilogue warps -> TMA
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int num_tiles = (n + kBN - 1) / kBN;
@@ -280,13 +291,20 @@ __global__ void __launch_bounds__(kAPThreads, 1)
     if (SPLIT == 3) tc::tma_prefetch_desc(&tm_lo);
     for (int s = 0; s < stages; ++s) {
       tc::mbar_init(full + s, 1);
-      tc::mbar_init(empty + s, 5);
+      tc::mbar_init(empty + s, KB == 0 ? 1 : 5);
     }
     for (int b = 0; b < 2; ++b) {
       tc::mbar_init(tfull + b, 1);
       tc::mbar_init(tempty + b, 4);
     }
-    tc::mbar_init(afull, 1);
+    if constexpr (KB == 0) {
+      for (int i = 0; i < kNrmSlots; ++i) {
+        tc::mbar_init(nfull + i, 1);
+        tc::mbar_init(nempty + i, 4);
+      }
+    } else {
+      tc::mbar_init(afull, 1);
+    }
     tc::fence_barrier_init();
   }
   if (warp == 1) {
@@ -300,7 +318,31 @@ __global__ void __launch_bounds__(kAPThreads, 1)
 
   if (warp == 0) {
     // ================= TMA producer =================
-    if (lane == 0) {
+    if constexpr (KB == 0) {
+      // (tile, k-block) in order; the stage counter runs over k-blocks across tiles
+      if (lane == 0) {
+        int s = 0;
+        uint32_t ph = 0;
+        for (int jt = 0; jt < num_tiles; ++jt) {
+          const int ns = jt % kNrmSlots;
+          tc::mbar_wait_backoff(nempty + ns, ((jt / kNrmSlots) & 1) ^ 1);
+          tc::mbar_arrive_expect_tx(nfull + ns, kBN * 4);
+          tc::bulk_load_1d(smem + L.nrm + ns * kBN * 4, nrm + (size_t)jt * kBN, kBN * 4, nfull + ns);
+          for (int kb = 0; kb < kblocks; ++kb, (++s == stages) ? (s = 0, ph ^= 1) : 0) {
+            tc::mbar_wait_backoff(empty + s, ph ^ 1);
+            tc::mbar_arrive_expect_tx(full + s, L.b_stage_bytes);
+            uint8_t* st = smem + L.b0 + s * L.b_stage_bytes;       // A_hi | A_lo | B_hi | B_lo
+            uint8_t* sb = st + (SPLIT == 3 ? 2 : 1) * kBM * 128;
+            for (int half = 0; half < 2; ++half) {
+              tc::tma_load_2d(st + half * 64 * 128, &tm_hi, full + s, kb * 32, row0 + half * 64);
+              if (SPLIT == 3) tc::tma_load_2d(st + (kBM + half * 64) * 128, &tm_lo, full + s, kb * 32, row0 + half * 64);
+            }
+            tc::tma_load_2d(sb, &tm_hi, full + s, kb * 32, jt * kBN);
+            if (SPLIT == 3) tc::tma_load_2d(sb + kBN * 128, &tm_lo, full + s, kb * 32, jt * kBN);
+          }
+        }
+      }
+    } else if (lane == 0) {
       const uint32_t a_bytes = KB * kBM * 128 * (SPLIT == 3 ? 2 : 1);
       tc::mbar_arrive_expect_tx(afull, a_bytes);
       for (int kb = 0; kb < KB; ++kb)
@@ -324,7 +366,40 @@ __global__ void __launch_bounds__(kAPThreads, 1)
     }
   } else if (warp == 1) {
     // ================= MMA issuer =================
-    if (lane == 0) {
+    if constexpr (KB == 0) {
+      if (lane == 0) {
+        constexpr uint32_t idesc = tc::idesc_tf32(kBM, kBN);
+        int s = 0;
+        uint32_t ph = 0;
+        for (int jt = 0; jt < num_tiles; ++jt) {
+          const int buf = jt & 1;
+          const uint32_t bph = (jt >> 1) & 1;
+          const uint32_t d_tmem = tmem_base + buf * kBN;
+          tc::mbar_wait_backoff(tempty + buf, bph ^ 1);
+          uint32_t acc = 0;
+          for (int kb = 0; kb < kblocks; ++kb, (++s == stages) ? (s = 0, ph ^= 1) : 0) {
+            tc::mbar_wait_backoff(full + s, ph);
+            tc::fence_after_sync();
+            const uint32_t a_hi = tc::smem_u32(smem + L.b0 + s * L.b_stage_bytes);
+            const uint32_t a_lo = a_hi + kBM * 128;
+            const uint32_t b_hi = a_hi + (SPLIT == 3 ? 2 : 1) * kBM * 128;
+            const uint32_t b_lo = b_hi + kBN * 128;
+#pragma unroll
+            for (int sp = 0; sp < SPLIT; ++sp) {
+              const uint32_t a = (sp == 2) ? a_lo : a_hi;   // hi*hi, hi*lo, lo*hi
+              const uint32_t b = (sp == 1) ? b_lo : b_hi;
+#pragma unroll
+              for (int ks = 0; ks < 4; ++ks) {
+                tc::mma_tf32(d_tmem, tc::smem_desc_k128(a + ks * 32), tc::smem_desc_k128(b + ks * 32), idesc, acc);
+                acc = 1;
+              }
+            }
+            tc::mma_commit(empty + s);     // stage reusable once this k-block's MMAs retire
+          }
+          tc::mma_commit(tfull + buf);     // after the tile's last k-block: accumulator ready for the epilogue
+        }
+      }
+    } else if (lane == 0) {
       constexpr uint32_t idesc = tc::idesc_tf32(kBM, kBN);
       tc::mbar_wait_backoff(afull, 0);
       tc::fence_after_sync();
@@ -405,10 +480,14 @@ __global__ void __launch_bounds__(kAPThreads, 1)
     for (int jt = 0; jt < num_tiles; ++jt, (++s == stages) ? (s = 0, ph ^= 1) : 0) {
       const int buf = jt & 1;
       const uint32_t bph = (jt >> 1) & 1;
-      tc::mbar_wait(full + s, ph);      // column norms of this tile are in smem
+      // where this tile's column norms are: its key stage, or (KB = 0) its slot of the norm ring
+      const int ns = KB == 0 ? jt % kNrmSlots : s;
+      uint64_t* nbar_full = KB == 0 ? nfull + ns : full + s;
+      uint64_t* nbar_empty = KB == 0 ? nempty + ns : empty + s;
+      tc::mbar_wait(nbar_full, KB == 0 ? (uint32_t)(jt / kNrmSlots) & 1 : ph);   // column norms are in smem
       tc::mbar_wait(tfull + buf, bph);  // accumulator ready
       tc::fence_after_sync();
-      const float* nj = reinterpret_cast<const float*>(smem + L.nrm + s * kBN * 4);
+      const float* nj = reinterpret_cast<const float*>(smem + L.nrm + ns * kBN * 4);
       // the tile(s) that contain this CTA's own diagonal take the variant that pins d2(i,i) = 0 exactly
       const bool diag_tile = (jt * kBN < row0 + kBM) && (jt * kBN + kBN > row0);
 #pragma unroll 1
@@ -467,7 +546,7 @@ __global__ void __launch_bounds__(kAPThreads, 1)
       __syncwarp();
       if (lane == 0) {
         tc::mbar_arrive(tempty + buf);
-        tc::mbar_arrive(empty + s);
+        tc::mbar_arrive(nbar_empty);
       }
     }
     flush(__ballot_sync(0xffffffffu, qn > 0));
@@ -1039,7 +1118,7 @@ static int64_t ap_base_workspace(int32_t n, int32_t d) {
 
 extern "C" int64_t dggb_allpairs_workspace_bytes_rows(int32_t n, int32_t d, int32_t row_count, int32_t kc) {
   if (n < 0 || d <= 0 || row_count < 0 || kc <= 0) return DGGB_ERR_BAD_ARG;
-  const int parts = ap_choose_parts(row_count, n, kc);
+  const int parts = d > 128 ? 1 : ap_choose_parts(row_count, n, kc);   // the streamed shape runs unsplit
   return ap_base_workspace(n, d) + (parts > 1 ? (int64_t)parts * row_count * kc * 8 : 0);
 }
 
@@ -1067,7 +1146,7 @@ extern "C" int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d
   if ((after_val == nullptr) != (after_idx == nullptr)) return DGGB_ERR_BAD_ARG;
   if (!z || !t || !workspace || !out_idx || !out_val || n <= 0 || d <= 0 || row_begin < 0 || row_count < 0 || kc <= 0)
     return DGGB_ERR_BAD_ARG;
-  if (d > 128 || kc > 64) return DGGB_ERR_BAD_SHAPE;
+  if (kc > 64) return DGGB_ERR_BAD_SHAPE;
   if (precision != 1 && precision != 3) return DGGB_ERR_UNSUPPORTED;
   if (workspace_bytes < dggb_allpairs_workspace_bytes(n, d)) return DGGB_ERR_WORKSPACE;
   if (row_count == 0) return DGGB_OK;
@@ -1089,6 +1168,9 @@ extern "C" int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d
   if (rc != DGGB_OK) return rc;
 
   const int kb = dpad / 32;
+  // d > 128: no kernel has room for the whole query tile, so v1's k-block-streamed instantiation (KB = 0) runs the call,
+  // unsplit, whatever DGGB_AP_V1 / DGGB_AP_PARTS say
+  const bool streamed = kb > 4;
   // ---- v2 (two epilogue groups, A in TMEM) whenever the second list/queue set fits: kc <= 32 ----
   const int nmode2 = noise ? 1 : (noise_scale != 0.f ? 2 : (out_rowsum ? 3 : 0));
   if (out_rowsum && nmode2 != 3) return DGGB_ERR_UNSUPPORTED;
@@ -1098,7 +1180,7 @@ extern "C" int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d
   // slots (flushed whenever anything is pending) to keep two stages + both groups' lists under 227 KB
   const bool big = (kb == 4 && precision == 3);
   const int qcap = big ? kChunk : kQCap, qflush = big ? 1 : kQFlush;
-  if (kc <= 32 && (want_v2 || big) && after_val == nullptr) {
+  if (!streamed && kc <= 32 && (want_v2 || big) && after_val == nullptr) {
     int st2 = 4;
     AP2Smem L2 = ap2_smem_layout(kb, precision, st2, kc, qcap);
     while (st2 > 2 && L2.total + 1024 > 227 * 1024) L2 = ap2_smem_layout(kb, precision, --st2, kc, qcap);
@@ -1188,9 +1270,10 @@ extern "C" int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d
     if (rc != DGGB_OK) return rc;
     return cont_pass(kc - 32, out_idx + 32, out_val + 32, out_val + 31, out_idx + 31, kc, nullptr);
   }
+  const int kbt = streamed ? 0 : kb;   // template KB
   int stages = 4;
-  APSmem L = ap_smem_layout(kb, precision, stages, kc);
-  while (stages > 2 && L.total + 1024 > 227 * 1024) L = ap_smem_layout(kb, precision, --stages, kc);
+  APSmem L = ap_smem_layout(kbt, precision, stages, kc);
+  while (stages > 2 && L.total + 1024 > 227 * 1024) L = ap_smem_layout(kbt, precision, --stages, kc);
   if (L.total + 1024 > 227 * 1024) return DGGB_ERR_BAD_SHAPE;
   const size_t smem_bytes = L.total + 1024;
   const int grid = (row_count + kBM - 1) / kBM;
@@ -1205,7 +1288,7 @@ extern "C" int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d
     if (e != cudaSuccess) return cuda_status(e);                                                                  \
     allpairs_topk_kernel<KB_, SP_, NM_><<<grid, kAPThreads, smem_bytes, st>>>(                                    \
         tm_hi, tm_lo, nrm, n, row_begin, row_count, t, noise, (long long)noise_ld, (unsigned long long)seed,      \
-        noise_scale, kc, stages, out_idx, out_val, inv_temp, out_rowsum, after_val, after_idx);                   \
+        noise_scale, kc, stages, out_idx, out_val, inv_temp, out_rowsum, after_val, after_idx, kb);               \
   } while (0)
 #define DGGB_AP_LAUNCH(KB_, SP_)                                                                                  \
   do {                                                                                                            \
@@ -1215,7 +1298,9 @@ extern "C" int dggb_allpairs_topk_after_fwd(const float* z, int32_t n, int32_t d
     else DGGB_AP_LAUNCH1(KB_, SP_, 3);                                                                            \
   } while (0)
 
-  if (kb == 1 && precision == 3) DGGB_AP_LAUNCH(1, 3);
+  if (streamed && precision == 3) DGGB_AP_LAUNCH(0, 3);
+  else if (streamed) DGGB_AP_LAUNCH(0, 1);
+  else if (kb == 1 && precision == 3) DGGB_AP_LAUNCH(1, 3);
   else if (kb == 1) DGGB_AP_LAUNCH(1, 1);
   else if (kb == 2 && precision == 3) DGGB_AP_LAUNCH(2, 3);
   else if (kb == 2) DGGB_AP_LAUNCH(2, 1);
